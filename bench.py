@@ -33,6 +33,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
@@ -385,6 +386,9 @@ def run_ours(args):
     barrier()
     ms_dev = max_over_ranks(e0.elapsed_time(e1))
     launches = eng.launches_per_step() * K
+    if args.dump_outputs and rank == 0:
+        # read back now: the e2e and profiling steps below update the parameters again
+        dump_outputs(args.dump_outputs, out, eng.get_params(), eng.get_grads())
 
     # ---------------- end to end through host buffers (`e2e`) ----------------
     for i in range(2):       # warm the copy path
@@ -503,6 +507,17 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(d, out, params, grads):
+    """What the last timed step returned to its caller: its scalars, the updated parameters and the gradient bucket
+    the update consumed (flat, float32, 16.6 MB each at the default shape), as <d>/<name>.npy."""
+    os.makedirs(d, exist_ok=True)
+    arrays = {k: np.float64(out[k]) for k in ("pi_loss", "baseline_loss", "entropy", "learning_rate", "grad_norm",
+                                              "total_loss", "step")}
+    arrays.update(params=params, grads=grads)
+    for k, v in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), v)
 
 
 # dram__bytes_read.sum + dram__bytes_write.sum per launch of vtrace_from_softmax_pipe_kernel at [65536,18,18], from the
@@ -674,7 +689,13 @@ def main():
                     help="impala = the headline IMPALA learner step (default); apex = the Ape-X DQN learner step "
                          "(BASELINE configs[3], tools/bench_apex.py); r2d2 = the R2D2 learner step (configs[4], "
                          "tools/bench_r2d2.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs (scalars, parameters, gradients) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "impala" or args.impl != "ours"):
+        ap.error("--dump-outputs is implemented for --workload impala --impl ours")
     if args.workload != "impala":
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         leg = __import__("bench_" + args.workload)

@@ -4,12 +4,11 @@
 is restated) and the reference checkout on ``sys.path`` and imports the reference's own modules
 (``agent/impala.py``, ``optimizer/vtrace.py``, ``model/impala_actor_critic.py``, ``agent/apex.py``, ``agent/r2d2.py``,
 ``distributed_queue/buffer_queue.py`` ...) exactly as they lie under ``/root/reference``: nothing is copied or edited.
-This is what pins ``oracle/impala_torch.py`` & co. to the reference itself: ``tests/test_oracle_refexec.py`` asserts
-that the restatements equal the executed reference (losses, V-trace taps, every gradient, the optimizer step) and
-``tests/golden/make_golden.py`` writes the committed golden vectors from the executed reference.
+This is what pins ``oracle/impala_torch.py`` & co. to the reference itself: ``tests/golden/make_golden.py`` writes
+the committed golden vectors from the executed reference, and ``tests/test_oracle_refexec.py`` asserts that the
+restatements equal them (losses, V-trace taps, every gradient, the optimizer step).
 
-The reference checkout exists only in the build container (``/root/reference``; override with ``DRL_REFERENCE_DIR``);
-on the GPU box the committed goldens stand in for it.
+``DRL_REFERENCE_DIR`` names the reference checkout; the tests do not need one.
 """
 import importlib
 import os

@@ -21,7 +21,6 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-STRIDE = 61
 ORDER = ("conv2d", "conv2d_1", "conv2d_2", "dense", "dense_1", "rnn/lstm_cell", "dense_2", "dense_3", "dense_4",
          "dense_5", "dense_6", "dense_7")
 NAMES = ("conv1", "conv2", "conv3", "emb1", "emb2", "lstm", "actor1", "actor2", "actor3", "critic1", "critic2", "critic3")
@@ -62,15 +61,17 @@ def impala_case(tf, impala, B, T, A, seed):
     for k, v in zip(("vs", "clipped_rho", "vs_plus_1", "pg_advantage", "first_policy", "first_value"), tv):
         rec[k] = v
     for n, g in zip(var, gv):
-        if g.size > 70000:
-            rec["gradsample_" + n] = g.ravel()[::STRIDE].astype(np.float32)
-            rec["gradl2_" + n] = np.float64(np.sqrt(np.sum(g.astype(np.float64) ** 2)))
-        else:
-            rec["grad_" + n] = g.astype(np.float32)
-    for n in var:
-        rec["paramsample_" + n] = sess.run(var[n]).ravel()[::STRIDE]
-        rec["rmssample_" + n] = sess.run(agent.optimizer.get_slot(var[n], "rms")).ravel()[::STRIDE]
+        s = rec["stride_" + n] = sample_stride(g.size)
+        rec["gradsample_" + n] = g.ravel()[::s].astype(np.float32)
+        rec["gradl2_" + n] = np.float64(np.sqrt(np.sum(g.astype(np.float64) ** 2)))
+        rec["paramsample_" + n] = sess.run(var[n]).ravel()[::s]
+        rec["rmssample_" + n] = sess.run(agent.optimizer.get_slot(var[n], "rms")).ravel()[::s]
     return rec
+
+
+def sample_stride(n, most=512):
+    """The sampling of make_golden.py: a stride that keeps at most ``most`` elements, odd."""
+    return -(-n // most) | 1
 
 
 def compare(rec, path, tol=1e-4):

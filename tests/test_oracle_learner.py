@@ -152,5 +152,7 @@ def test_golden_fixture_matches_oracle():
         assert abs(v - float(z[k])) < 1e-9 * abs(float(z[k]))
     assert abs(gn - float(z["grad_norm"])) < 1e-9 * gn
     np.testing.assert_allclose(out["vs"].numpy(), z["vs"], rtol=1e-9)
-    np.testing.assert_allclose(g["conv1.w"].numpy(), z["grad_conv1.w"], rtol=1e-4, atol=1e-9)
-    np.testing.assert_allclose(g["lstm.w"].numpy().ravel()[::61], z["gradsample_lstm.w"], rtol=1e-4, atol=1e-9)
+    for n in g:
+        s = int(z["stride_" + n])
+        np.testing.assert_allclose(g[n].numpy().ravel()[::s], z["gradsample_" + n], rtol=1e-4, atol=1e-9, err_msg=n)
+        np.testing.assert_allclose(np.sqrt(np.sum(g[n].numpy() ** 2)), float(z["gradl2_" + n]), rtol=1e-9, err_msg=n)
