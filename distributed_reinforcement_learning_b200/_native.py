@@ -246,3 +246,83 @@ def as_c(arr, dtype, shape=None, name="array"):
 
 def ptr(a):
     return C.c_void_p(a.ctypes.data)
+
+
+def _as_u8(done):
+    d = np.asarray(done)
+    if d.dtype == np.bool_:
+        return np.ascontiguousarray(d).view(np.uint8)      # bool is one byte, 0/1: no copy
+    return d.astype(np.uint8, copy=False)
+
+
+class NativeHandle:
+    """What every learner wrapper does the same way through its ``drl_<prefix>_*`` entry points: create and destroy
+    the handle, parameters without a scope argument, gradients, named buffers, the per-kernel profile and the step's
+    stream, time and launch count."""
+    _prefix = None
+
+    def _fn(self, name):
+        return getattr(lib, "drl_%s_%s" % (self._prefix, name))
+
+    def _open(self, cfg, num_slots):
+        self._h = C.c_void_p()
+        check(self._fn("create")(C.byref(cfg), C.byref(self._h)))
+        n = C.c_int64()
+        check(self._fn("param_count")(self._h, C.byref(n)))
+        self.param_count = int(n.value)
+        self.num_slots = int(num_slots)
+        self._keep = [None] * self.num_slots     # host arrays referenced by in-flight H2D copies
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            self._fn("destroy")(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def set_params(self, flat):
+        a = as_c(flat, np.float32, (self.param_count,), "params")
+        check(self._fn("set_params")(self._h, ptr(a), a.size))
+
+    def get_params(self):
+        a = np.empty(self.param_count, np.float32)
+        check(self._fn("get_params")(self._h, ptr(a), a.size))
+        return a
+
+    def get_grads(self):
+        a = np.empty(self.param_count, np.float32)
+        check(self._fn("get_grads")(self._h, ptr(a), a.size))
+        return a
+
+    def read_buffer(self, name, count):
+        a = np.empty(int(count), np.float32)
+        check(self._fn("read_buffer")(self._h, name.encode(), ptr(a), a.size))
+        return a
+
+    def profile_step(self, slot=0, max_kernels=128):
+        """One real step with a CUDA event before every launch -> [(kernel name, device ms)]."""
+        names = C.create_string_buffer(8192)
+        ms = np.zeros(max_kernels, np.float32)
+        cnt = C.c_int32()
+        check(self._fn("profile_step")(self._h, slot, names, len(names), ptr(ms), max_kernels, C.byref(cnt)))
+        nm = names.value.decode().split("\n") if cnt.value else []
+        return list(zip(nm, [float(x) for x in ms[:cnt.value]]))
+
+    def last_step_ms(self):
+        ms = C.c_float()
+        check(self._fn("last_step_ms")(self._h, C.byref(ms)))
+        return float(ms.value)
+
+    def launches_per_step(self):
+        n = C.c_int32()
+        check(self._fn("launches_per_step")(self._h, C.byref(n)))
+        return int(n.value)
+
+    def stream_ptr(self):
+        s = C.c_void_p()
+        check(self._fn("stream")(self._h, C.byref(s)))
+        return int(s.value or 0)

@@ -6,10 +6,14 @@ import numpy as np
 
 from . import _native as N
 from . import dp
-from .apex_learner import _as_u8
+from ._native import _as_u8
 
 
-class NativeA3CLearner:
+class NativeA3CLearner(dp.AdamLearner):
+    _prefix = "a3c"
+    set_params = N.NativeHandle.set_params      # one network: no `which`
+    get_params = N.NativeHandle.get_params
+
     def __init__(self, batch, num_action=4, input_shape=(84, 84, 4), discount_factor=0.997, start_learning_rate=1e-4,
                  end_learning_rate=0.0, learning_frame=1000000000, baseline_loss_coef=1.0, entropy_coef=0.05,
                  gradient_clip_norm=40.0, reward_clipping="abs_one", device=0, num_slots=2, use_cuda_graph=False,
@@ -23,52 +27,7 @@ class NativeA3CLearner:
                           float(learning_frame), baseline_loss_coef, entropy_coef, gradient_clip_norm,
                           N.REWARD_CLIPPING[reward_clipping], int(device), int(num_slots), int(bool(use_cuda_graph)),
                           int(math_mode))
-        self._h = C.c_void_p()
-        N.check(N.lib.drl_a3c_create(C.byref(cfg), C.byref(self._h)))
-        n = C.c_int64()
-        N.check(N.lib.drl_a3c_param_count(self._h, C.byref(n)))
-        self.param_count = int(n.value)
-        self.num_slots = int(num_slots)
-        self._keep = [None] * self.num_slots
-        self._dp = dp.BucketAllReduce("a3c", self._h, int(device))
-
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            N.lib.drl_a3c_destroy(self._h)
-            self._h = C.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def set_params(self, flat):
-        a = N.as_c(flat, np.float32, (self.param_count,), "params")
-        N.check(N.lib.drl_a3c_set_params(self._h, N.ptr(a), a.size))
-
-    def get_params(self):
-        a = np.empty(self.param_count, np.float32)
-        N.check(N.lib.drl_a3c_get_params(self._h, N.ptr(a), a.size))
-        return a
-
-    def set_opt_state(self, m, v, step, beta1_power=0.9, beta2_power=0.999):
-        am = N.as_c(m, np.float32, (self.param_count,), "m")
-        av = N.as_c(v, np.float32, (self.param_count,), "v")
-        N.check(N.lib.drl_a3c_set_opt_state(self._h, N.ptr(am), N.ptr(av), am.size, int(step), float(beta1_power),
-                                            float(beta2_power)))
-
-    def get_opt_state(self):
-        m = np.empty(self.param_count, np.float32)
-        v = np.empty(self.param_count, np.float32)
-        st, b1, b2 = C.c_int64(), C.c_float(), C.c_float()
-        N.check(N.lib.drl_a3c_get_opt_state(self._h, N.ptr(m), N.ptr(v), m.size, C.byref(st), C.byref(b1), C.byref(b2)))
-        return dict(m=m, v=v, step=int(st.value), beta1_power=float(b1.value), beta2_power=float(b2.value))
-
-    def get_grads(self):
-        a = np.empty(self.param_count, np.float32)
-        N.check(N.lib.drl_a3c_get_grads(self._h, N.ptr(a), a.size))
-        return a
+        self._open(cfg, num_slots, int(device))
 
     def stage(self, slot, state, next_state, previous_action, action, reward, done):
         B = self.B
@@ -79,11 +38,7 @@ class NativeA3CLearner:
         self._keep[slot] = arrs
         N.check(N.lib.drl_a3c_stage(self._h, slot, *[N.ptr(a) for a in arrs]))
 
-    def step(self, slot=0):
-        if dp.distributed():
-            self._dp.step_async(slot)           # data parallel: see dp.py
-        else:
-            N.check(N.lib.drl_a3c_step_async(self._h, slot))
+    def wait(self):
         o = N.A3cOut()
         N.check(N.lib.drl_a3c_wait(self._h, C.byref(o)))
         return dict(pi_loss=o.pi_loss, baseline_loss=o.baseline_loss, entropy=o.entropy, learning_rate=o.learning_rate,
@@ -104,8 +59,3 @@ class NativeA3CLearner:
         out = [np.empty((B, self.A), np.float32), np.empty(B, np.float32), np.empty(B, np.float32), np.empty(B, np.float32)]
         N.check(N.lib.drl_a3c_taps(self._h, *[N.ptr(a) for a in out]))
         return dict(policy=out[0], value=out[1], next_value=out[2], advantage=out[3])
-
-    def read_buffer(self, name, count):
-        a = np.empty(int(count), np.float32)
-        N.check(N.lib.drl_a3c_read_buffer(self._h, name.encode(), N.ptr(a), a.size))
-        return a

@@ -11,18 +11,14 @@ import numpy as np
 
 from . import _native as N
 from . import dp
-
-MAIN, TARGET = 0, 1
-
-
-def _as_u8(done):
-    d = np.asarray(done)
-    if d.dtype == np.bool_:
-        return np.ascontiguousarray(d).view(np.uint8)
-    return d.astype(np.uint8, copy=False)
+from ._native import _as_u8
+from .dp import MAIN, TARGET  # noqa: F401  (the `which` of set_params / get_params)
 
 
-class NativeApexLearner:
+class NativeApexLearner(dp.AdamLearner):
+    _prefix = "apex"
+    _Out = N.ApexOut
+
     def __init__(self, batch, num_action=4, input_shape=(84, 84, 4), discount_factor=0.99, gradient_clip_norm=40.0,
                  reward_clipping="abs_one", start_learning_rate=1e-4, end_learning_rate=0.0,
                  learning_frame=100000000000000, device=0, num_slots=2, use_cuda_graph=False, math_mode=0):
@@ -35,54 +31,7 @@ class NativeApexLearner:
         cfg = N.ApexConfig(self.B, h, w, c, self.A, discount_factor, start_learning_rate, end_learning_rate,
                            float(learning_frame), gradient_clip_norm, clip, self.device, int(num_slots),
                            int(bool(use_cuda_graph)), int(math_mode))
-        self._h = C.c_void_p()
-        N.check(N.lib.drl_apex_create(C.byref(cfg), C.byref(self._h)))
-        n = C.c_int64()
-        N.check(N.lib.drl_apex_param_count(self._h, C.byref(n)))
-        self.param_count = int(n.value)
-        self.num_slots = int(num_slots)
-        self._keep = [None] * self.num_slots
-        self._dp = dp.BucketAllReduce("apex", self._h, self.device)
-
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            N.lib.drl_apex_destroy(self._h)
-            self._h = C.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    # ---- parameters / optimizer state -------------------------------------------------
-    def set_params(self, flat, which=MAIN):
-        a = N.as_c(flat, np.float32, (self.param_count,), "params")
-        N.check(N.lib.drl_apex_set_params(self._h, int(which), N.ptr(a), a.size))
-
-    def get_params(self, which=MAIN):
-        a = np.empty(self.param_count, np.float32)
-        N.check(N.lib.drl_apex_get_params(self._h, int(which), N.ptr(a), a.size))
-        return a
-
-    def set_opt_state(self, m, v, step, beta1_power=0.9, beta2_power=0.999):
-        am = N.as_c(m, np.float32, (self.param_count,), "m")
-        av = N.as_c(v, np.float32, (self.param_count,), "v")
-        N.check(N.lib.drl_apex_set_opt_state(self._h, N.ptr(am), N.ptr(av), am.size, int(step), float(beta1_power),
-                                             float(beta2_power)))
-
-    def get_opt_state(self):
-        m = np.empty(self.param_count, np.float32)
-        v = np.empty(self.param_count, np.float32)
-        st, b1, b2 = C.c_int64(), C.c_float(), C.c_float()
-        N.check(N.lib.drl_apex_get_opt_state(self._h, N.ptr(m), N.ptr(v), m.size, C.byref(st), C.byref(b1),
-                                             C.byref(b2)))
-        return dict(m=m, v=v, step=int(st.value), beta1_power=float(b1.value), beta2_power=float(b2.value))
-
-    def get_grads(self):
-        a = np.empty(self.param_count, np.float32)
-        N.check(N.lib.drl_apex_get_grads(self._h, N.ptr(a), a.size))
-        return a
+        self._open(cfg, num_slots, self.device)
 
     def target_to_main(self):
         """agent/apex.py:78-79: assigns target <- main (sic)."""
@@ -106,24 +55,6 @@ class NativeApexLearner:
     @staticmethod
     def _out(o):
         return dict(loss=o.loss, learning_rate=o.learning_rate, grad_norm=o.grad_norm, step=o.step)
-
-    def step(self, slot=0):
-        """-> (scalars dict, td_error [B]) of agent/apex.py:139-151.  With torch.distributed initialised (world > 1) the
-        step is data parallel: see dp.py."""
-        self.step_async(slot)
-        return self.wait()
-
-    def step_async(self, slot=0):
-        if dp.distributed():
-            self._dp.step_async(slot)
-        else:
-            N.check(N.lib.drl_apex_step_async(self._h, slot))
-
-    def wait(self):
-        o = N.ApexOut()
-        td = np.empty(self.B, np.float32)
-        N.check(N.lib.drl_apex_wait(self._h, C.byref(o), N.ptr(td)))
-        return self._out(o), td
 
     def td_error(self, state, next_state, previous_action, action, reward, done):
         """agent/apex.py:116-133 for n <= batch transitions."""
@@ -149,31 +80,3 @@ class NativeApexLearner:
         N.check(N.lib.drl_apex_taps(self._h, *[N.ptr(a) for a in out]))
         return dict(main_q=out[0], next_main_q=out[1], target_q=out[2], target_value=out[3],
                     state_action_value=out[4])
-
-    def read_buffer(self, name, count):
-        a = np.empty(int(count), np.float32)
-        N.check(N.lib.drl_apex_read_buffer(self._h, name.encode(), N.ptr(a), a.size))
-        return a
-
-    def profile_step(self, slot=0, max_kernels=128):
-        names = C.create_string_buffer(8192)
-        ms = np.zeros(max_kernels, np.float32)
-        cnt = C.c_int32()
-        N.check(N.lib.drl_apex_profile_step(self._h, slot, names, len(names), N.ptr(ms), max_kernels, C.byref(cnt)))
-        nm = names.value.decode().split("\n") if cnt.value else []
-        return list(zip(nm, [float(x) for x in ms[:cnt.value]]))
-
-    def last_step_ms(self):
-        ms = C.c_float()
-        N.check(N.lib.drl_apex_last_step_ms(self._h, C.byref(ms)))
-        return float(ms.value)
-
-    def launches_per_step(self):
-        n = C.c_int32()
-        N.check(N.lib.drl_apex_launches_per_step(self._h, C.byref(n)))
-        return int(n.value)
-
-    def stream_ptr(self):
-        s = C.c_void_p()
-        N.check(N.lib.drl_apex_stream(self._h, C.byref(s)))
-        return int(s.value or 0)

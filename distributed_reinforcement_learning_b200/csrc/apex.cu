@@ -7,50 +7,28 @@
 // over the B rows s'.  The attention_CNN and the action embedding are the same layers as IMPALA's, so they run
 // through the same gather-GEMM kernels (layer_defs.cuh); the two streams of the dueling head share their input
 // concat = [a3 | emb(prev_a)] (K = 3392), so their first layers are one split-K GEMM with N = 2 x 256.
-#include <string.h>
-
-#include <string>
-#include <mutex>
-#include <vector>
-
-#include "layer_defs.cuh"
+#include "adam_learner.cuh"
 
 namespace drl {
 
 // Offsets (in floats) inside the padded flat vectors of ONE network; same conventions as ParamLayout (kernels.h):
 // TF variable order, every bias directly behind its kernel and padded to 4 floats.
-struct ApexLayout {
+struct ApexLayout : FlatLayout<22> {
   int A;
   int64_t conv1_w, conv1_b, conv2_w, conv2_b, conv3_w, conv3_b;
   int64_t emb1_w, emb1_b, emb2_w, emb2_b;
   int64_t value1_w, value1_b, value2_w, value2_b, value3_w, value3_b;
   int64_t mean1_w, mean1_b, mean2_w, mean2_b, mean3_w, mean3_b;
-  int64_t padded_total, packed_total;
-  static constexpr int kNumTensors = 22;
-  int64_t packed_off[kNumTensors], padded_off[kNumTensors], count[kNumTensors];
   void init(int num_action) {
     A = num_action;
     const int64_t CAT = Geo::FLAT + Geo::EMB;
-    const int64_t sizes[kNumTensors] = {
-        8 * 8 * 4 * 32, 32, 4 * 4 * 32 * 64, 64, 3 * 3 * 64 * 64, 64,
-        (int64_t)A * 256, 256, 256 * 256, 256,
-        CAT * 256, 256, 256 * 256, 256, 256 * (int64_t)A, A,
-        CAT * 256, 256, 256 * 256, 256, 256, 1};
-    int64_t po = 0, pk = 0;
-    for (int i = 0; i < kNumTensors; ++i) {
-      count[i] = sizes[i];
-      packed_off[i] = pk;
-      padded_off[i] = po;
-      pk += sizes[i];
-      po += sizes[i];
-      if (i & 1) po = (po + 3) / 4 * 4;
-    }
-    packed_total = pk;
-    padded_total = (po + 3) / 4 * 4;
-    int64_t* f[kNumTensors] = {&conv1_w, &conv1_b, &conv2_w, &conv2_b, &conv3_w, &conv3_b, &emb1_w, &emb1_b,
-                               &emb2_w, &emb2_b, &value1_w, &value1_b, &value2_w, &value2_b, &value3_w, &value3_b,
-                               &mean1_w, &mean1_b, &mean2_w, &mean2_b, &mean3_w, &mean3_b};
-    for (int i = 0; i < kNumTensors; ++i) *f[i] = padded_off[i];
+    place({8 * 8 * 4 * 32, 32, 4 * 4 * 32 * 64, 64, 3 * 3 * 64 * 64, 64,
+           (int64_t)A * 256, 256, 256 * 256, 256,
+           CAT * 256, 256, 256 * 256, 256, 256 * (int64_t)A, A,
+           CAT * 256, 256, 256 * 256, 256, 256, 1},
+          {&conv1_w, &conv1_b, &conv2_w, &conv2_b, &conv3_w, &conv3_b, &emb1_w, &emb1_b, &emb2_w, &emb2_b, &value1_w,
+           &value1_b, &value2_w, &value2_b, &value3_w, &value3_b, &mean1_w, &mean1_b, &mean2_w, &mean2_b, &mean3_w,
+           &mean3_b});
   }
 };
 
@@ -232,101 +210,6 @@ __global__ void __launch_bounds__(256) a3c_loss_kernel(A3cArgs a) {
     a.loss[1] = t1 * inv_n;
     a.loss[2] = t2 * inv_n;
   }
-}
-
-// ------------------------------------------------------------------------------------------
-// Tail of the train op (agent/apex.py:70-75) with TF 1.14 semantics:
-//   lr    = polynomial_decay(start, global_step, decay_steps, end)      (float32, pre-increment step)
-//   g    <- g * clip * min(1/||g||, 1/clip)                              (clip_by_global_norm over the main variables;
-//                                                                         the target variables have gradient None)
-//   alpha = lr * sqrt(1 - beta2_power) / (1 - beta1_power)               (ApplyAdam, float32)
-//   m    += (g - m)(1 - beta1) ; v += (g^2 - v)(1 - beta2) ; w -= m * alpha / (sqrt(v) + eps)
-//   beta powers *= beta ; global_step += 1
-// Two launches: (1) partial squared norms + the scalars, (2) every block re-reduces the partials in fixed order.
-// ------------------------------------------------------------------------------------------
-constexpr float kBeta1 = 0.9f, kBeta2 = 0.999f, kAdamEps = 1e-8f;
-
-__global__ void __launch_bounds__(256) adam_prepare_kernel(AdamState o) {
-  pdl_prologue();
-  __shared__ float red[8];
-  const int64_t n4 = o.n / 4;
-  const float4* g4 = reinterpret_cast<const float4*>(o.grads);
-  float acc = 0.f;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
-    const float4 v = g4[i];
-    acc = fmaf(v.x, v.x, acc); acc = fmaf(v.y, v.y, acc); acc = fmaf(v.z, v.z, acc); acc = fmaf(v.w, v.w, acc);
-  }
-  acc = warp_sum(acc);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) s += red[i];
-    o.norm_partials[blockIdx.x] = s;
-    if (blockIdx.x == 0) {
-      const long long step = *o.step;
-      const float decay = (float)o.learning_frame;
-      const float gs = fminf((float)step, decay);
-      const float p = gs / decay;
-      const float lr = (o.start_lr - o.end_lr) * (1.0f - p) + o.end_lr;
-      const float b1 = *o.b1p, b2 = *o.b2p;
-      *o.lr_cur = lr;
-      *o.alpha = lr * sqrtf(1.0f - b2) / (1.0f - b1);
-      *o.b1p = b1 * kBeta1;
-      *o.b2p = b2 * kBeta2;
-      *o.step = step + 1;
-    }
-  }
-}
-
-__global__ void __launch_bounds__(256) adam_apply_kernel(AdamState o) {
-  pdl_prologue();
-  __shared__ float red[8];
-  __shared__ float s_scale;
-  float acc = 0.f;
-  for (int i = threadIdx.x; i < o.nblk; i += blockDim.x) acc += o.norm_partials[i];
-  acc = warp_sum(acc);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) s += red[i];
-    const float norm = sqrtf(s) * o.grad_scale;
-    s_scale = ((o.clip_norm > 0.f) ? o.clip_norm * fminf(1.0f / norm, 1.0f / o.clip_norm) : 1.0f) * o.grad_scale;
-    if (blockIdx.x == 0) {
-      o.out[0] = o.loss[0] * o.grad_scale; o.out[1] = *o.lr_cur; o.out[2] = norm;
-      o.out[3] = o.loss[1] * o.grad_scale; o.out[4] = o.loss[2] * o.grad_scale;          // A3C: baseline loss, entropy (zero for the DQN learners)
-      const long long st = *o.step;
-      o.out[6] = __int_as_float((int)(st & 0xffffffffll));
-      o.out[7] = __int_as_float((int)(st >> 32));
-    }
-  }
-  __syncthreads();
-  const float scale = s_scale;
-  const float alpha = *o.alpha;
-  const int64_t n4 = o.n / 4;
-  const float4* g4 = reinterpret_cast<const float4*>(o.grads);
-  float4* w4 = reinterpret_cast<float4*>(o.params);
-  float4* m4 = reinterpret_cast<float4*>(o.m);
-  float4* v4 = reinterpret_cast<float4*>(o.v);
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
-    const float4 g = g4[i];
-    float4 m = m4[i], v = v4[i], w = w4[i];
-    float gg;
-    gg = g.x * scale; m.x += (gg - m.x) * (1.0f - kBeta1); v.x += (gg * gg - v.x) * (1.0f - kBeta2); w.x -= (m.x * alpha) / (sqrtf(v.x) + kAdamEps);
-    gg = g.y * scale; m.y += (gg - m.y) * (1.0f - kBeta1); v.y += (gg * gg - v.y) * (1.0f - kBeta2); w.y -= (m.y * alpha) / (sqrtf(v.y) + kAdamEps);
-    gg = g.z * scale; m.z += (gg - m.z) * (1.0f - kBeta1); v.z += (gg * gg - v.z) * (1.0f - kBeta2); w.z -= (m.z * alpha) / (sqrtf(v.z) + kAdamEps);
-    gg = g.w * scale; m.w += (gg - m.w) * (1.0f - kBeta1); v.w += (gg * gg - v.w) * (1.0f - kBeta2); w.w -= (m.w * alpha) / (sqrtf(v.w) + kAdamEps);
-    m4[i] = m; v4[i] = v; w4[i] = w;
-  }
-}
-
-int adam_step(cudaStream_t s, const AdamState& o) {
-  DRL_CUDA_CHECK((launch_k(adam_prepare_kernel, o.nblk, 256, 0, s, o)));
-  DRL_CUDA_CHECK((launch_k(adam_apply_kernel, o.nblk, 256, 0, s, o)));
-  return DRL_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -540,118 +423,34 @@ static int apex_backward(const Streams& st, const ApexLayout& pl, const float* P
 }
 
 struct ApexSlot {
-  uint8_t* base = nullptr;
   uint8_t* frames = nullptr;   // [2B][84,84,4]: state rows, then next_state rows
   int32_t* pa2 = nullptr;      // [2B]: previous_action, then action (the embedding input of the rows s')
   float* reward = nullptr;     // [B]
   uint8_t* done = nullptr;     // [B]
   float* weight = nullptr;     // [B]
-  cudaEvent_t staged = nullptr, consumed = nullptr;
-  bool has_data = false;
 };
 
 }  // namespace drl
 
 using namespace drl;
 
-struct drl_apex {
-  std::recursive_mutex mu;   // every C-ABI entry point locks the handle (actor threads call parameter_sync -> get_params
-                             // on the learner's handle while the learner thread trains; ctypes drops the GIL)
+struct drl_apex : AdamLearner {
   drl_apex_config cfg{};
-  int B = 0, A = 0, mode = 2;
+  int A = 0;
   ApexLayout pl{};
-  cudaStream_t compute = nullptr, copy = nullptr, side = nullptr;
-  cudaEvent_t ev_start = nullptr, ev_stop = nullptr, ev_done = nullptr;
-  cudaEvent_t fj[8] = {};
-  // the target scope's forward is independent of the main scope's: it runs on its own stream pair beside it
-  cudaStream_t tmain = nullptr, tside = nullptr;
-  cudaEvent_t tfj[8] = {}, ev_tfork = nullptr, ev_tjoin = nullptr;
-  bool par = true;
-  float *params = nullptr, *target = nullptr, *adam_m = nullptr, *adam_v = nullptr, *grads = nullptr;
   ApexActs act{}, tact{};
   ApexBwd bwd{};
-  WeightImages wi{}, twi{};
-  bool main_images_stale = true, target_images_stale = true;
   float *main_q = nullptr, *next_main_q = nullptr, *target_q = nullptr, *target_value = nullptr, *sav = nullptr,
-        *td_dev = nullptr, *loss = nullptr;
-  int last_n = 0;              // rows of the most recent step / td_error call (taps, read_buffer)
+        *td_dev = nullptr;
   // A3C runs on the same body (drl_a3c_*): no target scope, the loss kernel above, three loss scalars
   int algo = 0;                // 0 = Ape-X DQN, 1 = A3C
   float a3c_baseline_coef = 0.f, a3c_entropy_coef = 0.f;
   int a3c_clip = 0;
   float* adv = nullptr;        // [B] advantage tap
-  AdamState opt{};
-  long long* d_step = nullptr;
-  float *d_lr = nullptr, *d_alpha = nullptr, *d_b1p = nullptr, *d_b2p = nullptr;
-  float *h_out = nullptr, *d_out = nullptr;     // mapped pinned [num_slots][8]
-  float *h_td = nullptr, *d_td = nullptr;       // mapped pinned [num_slots][B]
-  float* h_flat = nullptr;
-  float* h_ones = nullptr;                      // pinned [B] of 1.0f (unit importance weights)
-  std::vector<ApexSlot> slots;                  // num_slots training slots + 1 scratch slot for the synchronous calls
-  std::vector<void*> allocs;
-  std::vector<cudaGraphExec_t> graph_step;
-  bool pending = false;
-  int last_slot = 0;
-  int launches = 0;
+  std::vector<ApexSlot> slots; // payloads of AdamLearner::sync
 };
 
 namespace {
-
-template <class T>
-int dev_alloc(drl_apex* h, T** p, size_t count) {
-  void* q = nullptr;
-  DRL_CUDA_CHECK(cudaMalloc(&q, count * sizeof(T) + 256));
-  DRL_CUDA_CHECK(cudaMemset(q, 0, count * sizeof(T) + 256));
-  h->allocs.push_back(q);
-  *p = static_cast<T*>(q);
-  return DRL_OK;
-}
-size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-int check_handle(const drl_apex* h) {
-  if (!h) { set_error("null apex handle"); return DRL_ERR_INVALID; }
-  return DRL_OK;
-}
-int set_device(const drl_apex* h) {
-  DRL_CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  return DRL_OK;
-}
-
-int upload_flat(drl_apex* h, float* dev_padded, const float* host_packed) {
-  for (int64_t i = 0; i < h->pl.padded_total; ++i) h->h_flat[i] = 0.0f;
-  for (int i = 0; i < ApexLayout::kNumTensors; ++i)
-    memcpy(h->h_flat + h->pl.padded_off[i], host_packed + h->pl.packed_off[i], h->pl.count[i] * sizeof(float));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  DRL_CUDA_CHECK(cudaMemcpyAsync(dev_padded, h->h_flat, h->pl.padded_total * sizeof(float), cudaMemcpyHostToDevice, h->compute));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  return DRL_OK;
-}
-int download_flat(drl_apex* h, const float* dev_padded, float* host_packed) {
-  DRL_CUDA_CHECK(cudaMemcpyAsync(h->h_flat, dev_padded, h->pl.padded_total * sizeof(float), cudaMemcpyDeviceToHost, h->compute));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  for (int i = 0; i < ApexLayout::kNumTensors; ++i)
-    memcpy(host_packed + h->pl.packed_off[i], h->h_flat + h->pl.padded_off[i], h->pl.count[i] * sizeof(float));
-  return DRL_OK;
-}
-
-// stream pair of the target scope: its own pair when the step runs parallel, otherwise the main pair (serial)
-Streams target_streams_of(const drl_apex* h) {
-  Streams st;
-  st.main = h->par ? h->tmain : h->compute;
-  st.side = h->par ? h->tside : h->side;
-  for (int i = 0; i < 8; ++i) st.ev[i] = h->par ? h->tfj[i] : h->fj[i];
-  st.par = h->par;
-  return st;
-}
-
-Streams streams_of(const drl_apex* h) {
-  Streams st;
-  st.main = h->compute;
-  st.side = h->side;
-  for (int i = 0; i < 8; ++i) st.ev[i] = h->fj[i];
-  st.par = h->par;
-  return st;
-}
 
 int alloc_acts(drl_apex* h, ApexActs& a, int cap) {
   const size_t M = cap, A = h->A;
@@ -692,26 +491,16 @@ int enqueue_forward_td(drl_apex* h, const ApexSlot& sl, int n, bool train, float
     if (launches) *launches += 1;
     return DRL_OK;
   }
-  // the target forward has no dependence on the main forward: fork it onto its own stream pair first, join before the
-  // TD kernel (inside a captured step these become parallel branches of the graph)
-  if (h->par) {
-    DRL_CUDA_CHECK(cudaEventRecord(h->ev_tfork, h->compute));
-    DRL_CUDA_CHECK(cudaStreamWaitEvent(h->tmain, h->ev_tfork, 0));
-    pdl_break(h->tmain);
-    pdl_break(h->tside);
-  }
+  DRL_TRY(fork_target(h));
   DRL_TRY(apex_forward(tst, h->pl, h->target, h->twi, sl.frames + (size_t)n * Geo::FRAME, sl.pa2 + n, h->tact, n, h->mode,
                        h->target_images_stale, false, true, launches));
   h->target_images_stale = false;
-  if (h->par) DRL_CUDA_CHECK(cudaEventRecord(h->ev_tjoin, h->tmain));
+  DRL_TRY(target_done(h));
   // rows [0, n) = s with previous_action, rows [n, 2n) = s' with action: one main-network forward covers both
   DRL_TRY(apex_forward(st, h->pl, h->params, h->wi, sl.frames, sl.pa2, h->act, 2 * n, h->mode, h->main_images_stale,
                        h->main_images_stale, false, launches));
   h->main_images_stale = false;
-  if (h->par) {
-    DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, h->ev_tjoin, 0));
-    pdl_break(h->compute);
-  }
+  DRL_TRY(join_target(h));
   TdArgs a{};
   a.vstream = h->act.vstream; a.mstream = h->act.mstream;
   a.tvstream = h->tact.vstream; a.tmstream = h->tact.mstream;
@@ -728,99 +517,12 @@ int enqueue_forward_td(drl_apex* h, const ApexSlot& sl, int n, bool train, float
   return DRL_OK;
 }
 
-int enqueue_step(drl_apex* h, int slot, int* launches) {
+// the step's forward passes, loss and backward pass (FwdBwd of the shell, adam_learner.cuh)
+int forward_backward(drl_apex* h, int slot, int* launches) {
   const ApexSlot& sl = h->slots[slot];
-  const int B = h->B;
-  DRL_TRY(enqueue_forward_td(h, sl, B, true, h->d_td + (size_t)slot * B, launches));
-  DRL_TRY(apex_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, sl.frames, sl.pa2, h->act, h->bwd, 2 * B, B,
-                        h->mode, launches));
-  pdl_break(h->compute);
-  AdamState o = h->opt;
-  o.out = h->d_out + 8 * slot;
-  prof_mark(h->compute, "optimizer(norm+adam)");
-  DRL_TRY(adam_step(h->compute, o));
-  prof_mark(h->compute, "end");
-  if (launches) *launches += 2;
-  return DRL_OK;
-}
-
-int run_step(drl_apex* h, int slot) {
-  ApexSlot& sl = h->slots[slot];
-  if (!sl.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, sl.staged, 0));
-  // the weight images of the main network follow its parameters, which change every step; the target images only
-  // change with target_to_main / set_params.  Inside a captured graph the main retile is always part of the step.
-  if (h->cfg.use_cuda_graph && h->target_images_stale && h->mode >= 2) {
-    // refresh the target images outside of the graph so that the captured step never contains them
-    DRL_TRY((launch_retile_b<64>(h->compute, PlainB{h->target + h->pl.conv2_w, 64, 0}, 64, 512, h->twi.img[1])));
-    DRL_TRY((launch_retile_b<64>(h->compute, PlainB{h->target + h->pl.conv3_w, 64, 0}, 64, 576, h->twi.img[2])));
-    h->target_images_stale = false;
-  }
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_start, h->compute));
-  h->main_images_stale = true;
-  if (h->cfg.use_cuda_graph) {
-    if (!h->graph_step[slot]) {
-      // eager pass of forward + TD first (sets the per-kernel attributes outside of capture; it does not change any
-      // state the captured pass depends on: parameters and optimizer state are only touched by the update)
-      DRL_TRY(enqueue_forward_td(h, sl, h->B, true, h->d_td + (size_t)slot * h->B, nullptr));
-      DRL_TRY(apex_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, sl.frames, sl.pa2, h->act, h->bwd,
-                            2 * h->B, h->B, h->mode, nullptr));
-      h->main_images_stale = true;
-      cudaGraph_t g = nullptr;
-      int cnt = 0;
-      DRL_CUDA_CHECK(cudaStreamBeginCapture(h->compute, cudaStreamCaptureModeThreadLocal));
-      int r = enqueue_step(h, slot, &cnt);
-      cudaError_t e = cudaStreamEndCapture(h->compute, &g);
-      if (r != DRL_OK) { if (g) cudaGraphDestroy(g); return r; }
-      if (e != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(e)); return DRL_ERR_CUDA; }
-      DRL_CUDA_CHECK(cudaGraphInstantiate(&h->graph_step[slot], g, 0));
-      cudaGraphDestroy(g);
-      h->launches = cnt;
-    }
-    DRL_CUDA_CHECK(cudaGraphLaunch(h->graph_step[slot], h->compute));
-  } else {
-    int cnt = 0;
-    DRL_TRY(enqueue_step(h, slot, &cnt));
-    h->launches = cnt;
-  }
-  h->main_images_stale = true;      // the update changed the main parameters
-  h->last_n = h->B;
-  h->last_slot = slot;
-  DRL_CUDA_CHECK(cudaEventRecord(sl.consumed, h->compute));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_stop, h->compute));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_done, h->compute));
-  h->pending = true;
-  return DRL_OK;
-}
-
-// data parallel: the step in two halves around the caller's all-reduce of the bucket (eager launches)
-int run_forward_backward(drl_apex* h, int slot) {
-  ApexSlot& sl = h->slots[slot];
-  if (!sl.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, sl.staged, 0));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_start, h->compute));
-  h->main_images_stale = true;
-  int cnt = 0;
-  DRL_TRY(enqueue_forward_td(h, sl, h->B, true, h->d_td + (size_t)slot * h->B, &cnt));
-  DRL_TRY(apex_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, sl.frames, sl.pa2, h->act, h->bwd, 2 * h->B, h->B,
-                        h->mode, &cnt));
-  h->launches = cnt + 2;
-  h->last_n = h->B;
-  h->last_slot = slot;
-  DRL_CUDA_CHECK(cudaEventRecord(sl.consumed, h->compute));
-  return DRL_OK;
-}
-int run_apply(drl_apex* h, float grad_scale) {
-  pdl_break(h->compute);
-  AdamState o = h->opt;
-  o.out = h->d_out + 8 * h->last_slot;
-  o.grad_scale = grad_scale;
-  DRL_TRY(adam_step(h->compute, o));
-  h->main_images_stale = true;
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_stop, h->compute));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_done, h->compute));
-  h->pending = true;
-  return DRL_OK;
+  DRL_TRY(enqueue_forward_td(h, sl, h->B, true, h->d_td + (size_t)slot * h->B, launches));
+  return apex_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, sl.frames, sl.pa2, h->act, h->bwd, 2 * h->B,
+                       h->B, h->mode, launches);
 }
 
 int stage_into(drl_apex* h, ApexSlot& s, cudaStream_t stream, int n, int row2, const uint8_t* state,
@@ -863,25 +565,9 @@ int drl_apex_create(const drl_apex_config* cfg, drl_apex** out) {
   h->B = cfg->batch; h->A = cfg->num_action;
   h->pl.init(h->A);
   int rc = [&]() -> int {
-    DRL_TRY(set_device(h));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->compute, cudaStreamNonBlocking));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->copy, cudaStreamNonBlocking));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking));
-    for (int i = 0; i < 8; ++i) DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->fj[i], cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->tmain, cudaStreamNonBlocking));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->tside, cudaStreamNonBlocking));
-    for (int i = 0; i < 8; ++i) DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->tfj[i], cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_tfork, cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_tjoin, cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaEventCreate(&h->ev_start));
-    DRL_CUDA_CHECK(cudaEventCreate(&h->ev_stop));
-    DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming));
-    const size_t B = h->B, A = h->A, NP = h->pl.padded_total;
-    DRL_TRY(dev_alloc(h, &h->params, NP));
-    DRL_TRY(dev_alloc(h, &h->target, NP));
-    DRL_TRY(dev_alloc(h, &h->adam_m, NP));
-    DRL_TRY(dev_alloc(h, &h->adam_v, NP));
-    DRL_TRY(dev_alloc(h, &h->grads, NP + 4));
+    const size_t B = h->B, A = h->A;
+    DRL_TRY(create_shell(h, B, AdamSchedule{cfg->start_learning_rate, cfg->end_learning_rate, cfg->learning_frame,
+                                            cfg->gradient_clip_norm}));
     DRL_TRY(alloc_acts(h, h->act, 2 * h->B));
     DRL_TRY(alloc_acts(h, h->tact, h->B));
     ApexBwd& b = h->bwd;
@@ -899,51 +585,14 @@ int drl_apex_create(const drl_apex_config* cfg, drl_apex** out) {
     DRL_TRY(dev_alloc(h, &b.wg_part, wg));
     DRL_TRY(dev_alloc(h, &b.wg_part2, wg));
     DRL_TRY(dev_alloc(h, &b.dcol, B * 81 * 512));
-    {
-      size_t wb[WeightImages::kCount];
-      weight_image_sizes(wb);
-      for (int i : {1, 2, 5, 6}) DRL_TRY(dev_alloc(h, &h->wi.img[i], wb[i]));
-      for (int i : {1, 2}) DRL_TRY(dev_alloc(h, &h->twi.img[i], wb[i]));
-    }
     DRL_TRY(dev_alloc(h, &h->main_q, B * A));
     DRL_TRY(dev_alloc(h, &h->next_main_q, B * A));
     DRL_TRY(dev_alloc(h, &h->target_q, B * A));
     DRL_TRY(dev_alloc(h, &h->target_value, B));
     DRL_TRY(dev_alloc(h, &h->sav, B));
     DRL_TRY(dev_alloc(h, &h->td_dev, B));
-    h->loss = h->grads + NP;     // the loss scalars ride in the tail of the gradient bucket (one all-reduce covers both)
     DRL_TRY(dev_alloc(h, &h->adv, B));
-    DRL_TRY(dev_alloc(h, &h->d_step, 1));
-    DRL_TRY(dev_alloc(h, &h->d_lr, 1));
-    DRL_TRY(dev_alloc(h, &h->d_alpha, 1));
-    DRL_TRY(dev_alloc(h, &h->d_b1p, 1));
-    DRL_TRY(dev_alloc(h, &h->d_b2p, 1));
-    {
-      const float b1 = kBeta1, b2 = kBeta2;
-      DRL_CUDA_CHECK(cudaMemcpy(h->d_b1p, &b1, 4, cudaMemcpyHostToDevice));
-      DRL_CUDA_CHECK(cudaMemcpy(h->d_b2p, &b2, 4, cudaMemcpyHostToDevice));
-    }
-    const size_t ns = h->cfg.num_slots;
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_out, ns * 8 * sizeof(float), cudaHostAllocMapped));
-    DRL_CUDA_CHECK(cudaHostGetDevicePointer((void**)&h->d_out, h->h_out, 0));
-    memset(h->h_out, 0, ns * 8 * sizeof(float));
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_td, ns * B * sizeof(float), cudaHostAllocMapped));
-    DRL_CUDA_CHECK(cudaHostGetDevicePointer((void**)&h->d_td, h->h_td, 0));
-    memset(h->h_td, 0, ns * B * sizeof(float));
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_flat, NP * sizeof(float), cudaHostAllocDefault));
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_ones, B * sizeof(float), cudaHostAllocDefault));
-    for (size_t i = 0; i < B; ++i) h->h_ones[i] = 1.0f;
-    AdamState& o = h->opt;
-    o.params = h->params; o.m = h->adam_m; o.v = h->adam_v; o.grads = h->grads; o.n = (int64_t)NP;
-    o.nblk = 148 * 4;
-    DRL_TRY(dev_alloc(h, &o.norm_partials, o.nblk));
-    o.step = h->d_step; o.lr_cur = h->d_lr; o.alpha = h->d_alpha; o.b1p = h->d_b1p; o.b2p = h->d_b2p;
-    o.out = h->d_out; o.loss = h->loss;
-    o.start_lr = cfg->start_learning_rate; o.end_lr = cfg->end_learning_rate; o.learning_frame = cfg->learning_frame;
-    o.clip_norm = cfg->gradient_clip_norm;
-    o.grad_scale = 1.0f;
-    h->slots.resize(ns + 1);
-    h->graph_step.assign(ns, nullptr);
+    h->slots.resize(h->sync.size());
     for (ApexSlot& s : h->slots) {
       size_t off = 0;
       const size_t o_fr = off; off = align_up(off + 2 * B * Geo::FRAME, 256);
@@ -951,200 +600,93 @@ int drl_apex_create(const drl_apex_config* cfg, drl_apex** out) {
       const size_t o_rw = off; off = align_up(off + B * 4, 256);
       const size_t o_dn = off; off = align_up(off + B, 256);
       const size_t o_wt = off; off = align_up(off + B * 4, 256);
-      DRL_TRY(dev_alloc(h, &s.base, off));
-      s.frames = s.base + o_fr;
-      s.pa2 = reinterpret_cast<int32_t*>(s.base + o_pa);
-      s.reward = reinterpret_cast<float*>(s.base + o_rw);
-      s.done = s.base + o_dn;
-      s.weight = reinterpret_cast<float*>(s.base + o_wt);
-      DRL_CUDA_CHECK(cudaEventCreateWithFlags(&s.staged, cudaEventDisableTiming));
-      DRL_CUDA_CHECK(cudaEventCreateWithFlags(&s.consumed, cudaEventDisableTiming));
+      uint8_t* base = nullptr;
+      DRL_TRY(dev_alloc(h, &base, off));
+      s.frames = base + o_fr;
+      s.pa2 = reinterpret_cast<int32_t*>(base + o_pa);
+      s.reward = reinterpret_cast<float*>(base + o_rw);
+      s.done = base + o_dn;
+      s.weight = reinterpret_cast<float*>(base + o_wt);
     }
     DRL_CUDA_CHECK(cudaDeviceSynchronize());
     return DRL_OK;
   }();
-  if (rc != DRL_OK) {
-    std::string keep = get_error();
-    drl_apex_destroy(h);
-    set_error("%s", keep.c_str());
-    return rc;
-  }
-  *out = h;
-  return DRL_OK;
+  return finish_create(h, rc, out);
 }
 
-int drl_apex_destroy(drl_apex* h) {
-  if (!h) return DRL_OK;
-  cudaSetDevice(h->cfg.device);
-  cudaDeviceSynchronize();
-  for (auto g : h->graph_step) if (g) cudaGraphExecDestroy(g);
-  for (ApexSlot& s : h->slots) {
-    if (s.staged) cudaEventDestroy(s.staged);
-    if (s.consumed) cudaEventDestroy(s.consumed);
-  }
-  for (void* p : h->allocs) cudaFree(p);
-  if (h->h_out) cudaFreeHost(h->h_out);
-  if (h->h_td) cudaFreeHost(h->h_td);
-  if (h->h_flat) cudaFreeHost(h->h_flat);
-  if (h->h_ones) cudaFreeHost(h->h_ones);
-  if (h->ev_start) cudaEventDestroy(h->ev_start);
-  if (h->ev_stop) cudaEventDestroy(h->ev_stop);
-  if (h->ev_done) cudaEventDestroy(h->ev_done);
-  for (int i = 0; i < 8; ++i) if (h->fj[i]) cudaEventDestroy(h->fj[i]);
-  for (int i = 0; i < 8; ++i) if (h->tfj[i]) cudaEventDestroy(h->tfj[i]);
-  if (h->ev_tfork) cudaEventDestroy(h->ev_tfork);
-  if (h->ev_tjoin) cudaEventDestroy(h->ev_tjoin);
-  if (h->tmain) cudaStreamDestroy(h->tmain);
-  if (h->tside) cudaStreamDestroy(h->tside);
-  if (h->side) cudaStreamDestroy(h->side);
-  if (h->compute) cudaStreamDestroy(h->compute);
-  if (h->copy) cudaStreamDestroy(h->copy);
-  cudaGetLastError();
-  delete h;
-  return DRL_OK;
-}
+int drl_apex_destroy(drl_apex* h) { return destroy_shell(h); }
 
 int drl_apex_param_count(const drl_apex* h, int64_t* n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (!n) { set_error("null argument"); return DRL_ERR_INVALID; }
   *n = h->pl.packed_total;
   return DRL_OK;
 }
-
 int drl_apex_set_params(drl_apex* h, int32_t which, const float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (which != DRL_APEX_MAIN && which != DRL_APEX_TARGET) { set_error("which must be DRL_APEX_MAIN or DRL_APEX_TARGET"); return DRL_ERR_INVALID; }
-  if (!host_flat || n != h->pl.packed_total) { set_error("set_params: expected %lld floats, got %lld", (long long)h->pl.packed_total, (long long)n); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_TRY(upload_flat(h, which == DRL_APEX_MAIN ? h->params : h->target, host_flat));
-  if (which == DRL_APEX_MAIN) h->main_images_stale = true; else h->target_images_stale = true;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return set_params(h, which, host_flat, n);
 }
 int drl_apex_get_params(drl_apex* h, int32_t which, float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (which != DRL_APEX_MAIN && which != DRL_APEX_TARGET) { set_error("which must be DRL_APEX_MAIN or DRL_APEX_TARGET"); return DRL_ERR_INVALID; }
-  if (!host_flat || n != h->pl.packed_total) { set_error("get_params: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return download_flat(h, which == DRL_APEX_MAIN ? h->params : h->target, host_flat);
+  DRL_ENTER(h);
+  return get_params(h, which, host_flat, n);
 }
-
 int drl_apex_set_opt_state(drl_apex* h, const float* host_m, const float* host_v, int64_t n, int64_t step,
                            float beta1_power, float beta2_power) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (!host_m || !host_v || n != h->pl.packed_total) { set_error("set_opt_state: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_TRY(upload_flat(h, h->adam_m, host_m));
-  DRL_TRY(upload_flat(h, h->adam_v, host_v));
-  long long st = step;
-  DRL_CUDA_CHECK(cudaMemcpy(h->d_step, &st, sizeof(st), cudaMemcpyHostToDevice));
-  DRL_CUDA_CHECK(cudaMemcpy(h->d_b1p, &beta1_power, 4, cudaMemcpyHostToDevice));
-  DRL_CUDA_CHECK(cudaMemcpy(h->d_b2p, &beta2_power, 4, cudaMemcpyHostToDevice));
-  return DRL_OK;
+  DRL_ENTER(h);
+  return set_opt_state(h, host_m, host_v, n, step, beta1_power, beta2_power);
 }
 int drl_apex_get_opt_state(drl_apex* h, float* host_m, float* host_v, int64_t n, int64_t* step, float* beta1_power,
                            float* beta2_power) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (n != h->pl.packed_total) { set_error("get_opt_state: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  if (host_m) DRL_TRY(download_flat(h, h->adam_m, host_m));
-  if (host_v) DRL_TRY(download_flat(h, h->adam_v, host_v));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  if (step) {
-    long long st = 0;
-    DRL_CUDA_CHECK(cudaMemcpy(&st, h->d_step, sizeof(st), cudaMemcpyDeviceToHost));
-    *step = st;
-  }
-  if (beta1_power) DRL_CUDA_CHECK(cudaMemcpy(beta1_power, h->d_b1p, 4, cudaMemcpyDeviceToHost));
-  if (beta2_power) DRL_CUDA_CHECK(cudaMemcpy(beta2_power, h->d_b2p, 4, cudaMemcpyDeviceToHost));
-  return DRL_OK;
+  DRL_ENTER(h);
+  return get_opt_state(h, host_m, host_v, n, step, beta1_power, beta2_power);
 }
 int drl_apex_get_grads(drl_apex* h, float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (!host_flat || n != h->pl.packed_total) { set_error("get_grads: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return download_flat(h, h->grads, host_flat);
+  DRL_ENTER(h);
+  return get_grads(h, host_flat, n);
 }
-
 int drl_apex_target_to_main(drl_apex* h) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  DRL_TRY(set_device(h));
-  DRL_CUDA_CHECK(cudaMemcpyAsync(h->target, h->params, h->pl.padded_total * sizeof(float), cudaMemcpyDeviceToDevice, h->compute));
-  pdl_break(h->compute);
-  h->target_images_stale = true;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return copy_main_to_target(h);
 }
 
 int drl_apex_stage(drl_apex* h, int32_t slot, const uint8_t* state, const uint8_t* next_state,
                    const int32_t* previous_action, const int32_t* action, const float* reward, const uint8_t* done,
                    const float* is_weight) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
+  DRL_ENTER(h);
   if (!state || !next_state || !previous_action || !action || !reward || !done) { set_error("stage: null input pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  ApexSlot& s = h->slots[slot];
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->copy, s.consumed, 0));
-  DRL_TRY(stage_into(h, s, h->copy, h->B, h->B, state, next_state, previous_action, action, reward, done, is_weight));
-  DRL_CUDA_CHECK(cudaEventRecord(s.staged, h->copy));
-  s.has_data = true;
-  return DRL_OK;
+  return stage_slot(h, slot, [&](cudaStream_t s) {
+    return stage_into(h, h->slots[slot], s, h->B, h->B, state, next_state, previous_action, action, reward, done,
+                      is_weight);
+  });
 }
 
 int drl_apex_step_async(drl_apex* h, int32_t slot) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return run_step(h, slot);
+  DRL_ENTER(h);
+  return run_step(h, slot, forward_backward);
 }
-
 int drl_apex_forward_backward(drl_apex* h, int32_t slot) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return run_forward_backward(h, slot);
+  DRL_ENTER(h);
+  return run_forward_backward(h, slot, forward_backward);
 }
 int drl_apex_grad_bucket(drl_apex* h, void** dev_ptr, int64_t* count) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (dev_ptr) *dev_ptr = h->grads;
-  if (count) *count = h->pl.padded_total + 4;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return grad_bucket(h, dev_ptr, count);
 }
 int drl_apex_apply(drl_apex* h, float grad_scale) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (!(grad_scale > 0.f)) { set_error("apply: grad_scale must be > 0"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
+  DRL_ENTER(h);
   return run_apply(h, grad_scale);
 }
 
 int drl_apex_wait(drl_apex* h, drl_apex_out* out, float* td_error) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (!h->pending) { set_error("wait: no step in flight"); return DRL_ERR_STATE; }
-  DRL_TRY(set_device(h));
-  h->pending = false;
-  DRL_CUDA_CHECK(cudaEventSynchronize(h->ev_done));
-  const float* r = h->h_out + 8 * h->last_slot;
+  DRL_ENTER(h);
+  const float* r = nullptr;
+  DRL_TRY(wait_step(h, td_error, &r));
   if (out) {
     out->loss = r[0];
     out->learning_rate = r[1];
     out->grad_norm = r[2];
-    uint32_t lo, hi;
-    memcpy(&lo, &r[6], 4);
-    memcpy(&hi, &r[7], 4);
-    out->step = (int64_t)(((uint64_t)hi << 32) | lo);
+    out->step = result_row_step(r);
   }
-  if (td_error) memcpy(td_error, h->h_td + (size_t)h->last_slot * h->B, (size_t)h->B * sizeof(float));
   return DRL_OK;
 }
 
@@ -1156,11 +698,9 @@ int drl_apex_step(drl_apex* h, int32_t slot, drl_apex_out* out, float* td_error)
 int drl_apex_td_error(drl_apex* h, int32_t n, const uint8_t* state, const uint8_t* next_state,
                       const int32_t* previous_action, const int32_t* action, const float* reward, const uint8_t* done,
                       float* td_error) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (n < 1 || n > h->B) { set_error("td_error: n must be in [1, %d]", h->B); return DRL_ERR_INVALID; }
   if (!state || !next_state || !previous_action || !action || !reward || !done || !td_error) { set_error("td_error: null pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   ApexSlot& s = h->slots[h->cfg.num_slots];      // scratch slot
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
   // rows [0, n) = s, rows [n, 2n) = s' (packed, so that one main-network forward covers both)
@@ -1184,16 +724,14 @@ int drl_apex_td_error(drl_apex* h, int32_t n, const uint8_t* state, const uint8_
   DRL_CUDA_CHECK((launch_k(apex_td_kernel, 1, 256, 0, h->compute, a)));
   DRL_CUDA_CHECK(cudaMemcpyAsync(td_error, h->td_dev, (size_t)n * 4, cudaMemcpyDeviceToHost, h->compute));
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  h->last_n = n;
+  h->last_rows = n;
   return DRL_OK;
 }
 
 int drl_apex_act(drl_apex* h, int32_t n, const uint8_t* state, const int32_t* previous_action, float* q_value) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (n < 1 || n > 2 * h->B) { set_error("act: n must be in [1, %d]", 2 * h->B); return DRL_ERR_INVALID; }
   if (!state || !previous_action || !q_value) { set_error("act: null pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   ApexSlot& s = h->slots[h->cfg.num_slots];
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
   DRL_TRY(stage_into(h, s, h->compute, n, n, state, nullptr, previous_action, nullptr, nullptr, nullptr, nullptr));
@@ -1208,18 +746,16 @@ int drl_apex_act(drl_apex* h, int32_t n, const uint8_t* state, const int32_t* pr
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
   for (int i = 0; i < n; ++i)
     for (int k = 0; k < A; ++k) q_value[(size_t)i * A + k] = v[(size_t)i * A + k] - m[i];   // model/apex_value.py:40
-  h->last_n = 0;
+  h->last_rows = 0;
   return DRL_OK;
 }
 
 int drl_apex_taps(drl_apex* h, float* main_q, float* next_main_q, float* target_q, float* target_value,
                   float* state_action_value) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  DRL_TRY(set_device(h));
-  if (h->last_n < 1) { set_error("taps: no step or td_error call has run"); return DRL_ERR_STATE; }
+  DRL_ENTER(h);
+  if (h->last_rows < 1) { set_error("taps: no step or td_error call has run"); return DRL_ERR_STATE; }
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  const size_t n = h->last_n, A = h->A;
+  const size_t n = h->last_rows, A = h->A;
   if (main_q) DRL_CUDA_CHECK(cudaMemcpy(main_q, h->main_q, n * A * 4, cudaMemcpyDeviceToHost));
   if (next_main_q) DRL_CUDA_CHECK(cudaMemcpy(next_main_q, h->next_main_q, n * A * 4, cudaMemcpyDeviceToHost));
   if (target_q) DRL_CUDA_CHECK(cudaMemcpy(target_q, h->target_q, n * A * 4, cudaMemcpyDeviceToHost));
@@ -1229,75 +765,38 @@ int drl_apex_taps(drl_apex* h, float* main_q, float* next_main_q, float* target_
 }
 
 int drl_apex_read_buffer(drl_apex* h, const char* name, float* host_dst, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (!name || !host_dst) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  if (h->last_n < 1) { set_error("read_buffer: no step or td_error call has run"); return DRL_ERR_STATE; }
-  const size_t Mb = h->last_n, M = 2 * Mb, A = h->A;
-  struct Ent { const char* nm; const float* p; size_t cnt; };
-  const Ent tab[] = {
+  if (h->last_rows < 1) { set_error("read_buffer: no step or td_error call has run"); return DRL_ERR_STATE; }
+  const size_t Mb = h->last_rows, M = 2 * Mb, A = h->A;
+  const NamedBuffer tab[] = {
       {"a1", h->act.a1, M * 400 * 32}, {"a2", h->act.a2, M * 81 * 64}, {"a3", h->act.a3, M * Geo::FLAT},
       {"emb", h->act.table, A * Geo::EMB}, {"e1", h->act.e1, A * Geo::EMB},
       {"hid1", h->act.hid1, 2 * M * Geo::HID}, {"hid2", h->act.hid2, 2 * M * Geo::HID},
       {"da3", h->bwd.da3, Mb * Geo::FLAT}, {"da2", h->bwd.da2, Mb * 81 * 64}, {"da1", h->bwd.da1, Mb * 400 * 32}};
-  for (const Ent& e : tab) {
-    if (strcmp(e.nm, name) == 0) {
-      if ((size_t)n != e.cnt) { set_error("read_buffer(%s): expected %zu floats, got %lld", name, e.cnt, (long long)n); return DRL_ERR_INVALID; }
-      DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-      DRL_CUDA_CHECK(cudaMemcpy(host_dst, e.p, e.cnt * sizeof(float), cudaMemcpyDeviceToHost));
-      return DRL_OK;
-    }
-  }
-  set_error("read_buffer: unknown buffer '%s'", name);
-  return DRL_ERR_INVALID;
+  return read_named_buffer(h->compute, tab, sizeof(tab) / sizeof(tab[0]), name, host_dst, n);
 }
 
 int drl_apex_profile_step(drl_apex* h, int32_t slot, char* names, int64_t names_len, float* ms, int32_t max_kernels,
                           int32_t* count) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  if (!names || !ms || !count) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  ApexSlot& sl = h->slots[slot];
-  if (!sl.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, sl.staged, 0));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  prof_begin();
-  const bool par_saved = h->par;
-  h->par = false;
-  h->main_images_stale = true;
-  int rc = enqueue_step(h, slot, nullptr);
-  h->par = par_saved;
-  h->main_images_stale = true;
-  h->last_n = h->B;
-  DRL_TRY(prof_end(h->compute, rc, names, names_len, ms, max_kernels, count));
-  h->pending = false;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return profile_step(h, slot, forward_backward, names, names_len, ms, max_kernels, count);
 }
 
 int drl_apex_last_step_ms(drl_apex* h, float* ms) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  if (!ms) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_CUDA_CHECK(cudaEventSynchronize(h->ev_stop));
-  DRL_CUDA_CHECK(cudaEventElapsedTime(ms, h->ev_start, h->ev_stop));
-  return DRL_OK;
+  DRL_ENTER(h);
+  return last_step_ms(h, ms);
 }
 
 int drl_apex_stream(drl_apex* h, void** stream) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (!stream) { set_error("null argument"); return DRL_ERR_INVALID; }
   *stream = h->compute;
   return DRL_OK;
 }
 
 int drl_apex_launches_per_step(const drl_apex* h, int32_t* n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (!n) { set_error("null argument"); return DRL_ERR_INVALID; }
   *n = h->launches;     // valid after the first step
   return DRL_OK;
@@ -1343,23 +842,20 @@ int drl_a3c_stage(drl_a3c* h, int32_t slot, const uint8_t* state, const uint8_t*
   return drl_apex_stage(h, slot, state, next_state, previous_action, action, reward, done, nullptr);
 }
 int drl_a3c_step_async(drl_a3c* h, int32_t slot) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (h->algo != 1) { set_error("not an A3C handle"); return DRL_ERR_INVALID; }
-  return drl_apex_step_async(h, slot);
+  return run_step(h, slot, forward_backward);
 }
 int drl_a3c_forward_backward(drl_a3c* h, int32_t slot) { return drl_apex_forward_backward(h, slot); }
 int drl_a3c_grad_bucket(drl_a3c* h, void** dev_ptr, int64_t* count) { return drl_apex_grad_bucket(h, dev_ptr, count); }
 int drl_a3c_apply(drl_a3c* h, float grad_scale) { return drl_apex_apply(h, grad_scale); }
 int drl_a3c_wait(drl_a3c* h, drl_a3c_out* out) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  drl_apex_out o{};
-  DRL_TRY(drl_apex_wait(h, &o, nullptr));
+  DRL_ENTER(h);
+  const float* r = nullptr;
+  DRL_TRY(wait_step(h, nullptr, &r));
   if (out) {
-    const float* r = h->h_out + 8 * h->last_slot;
     out->pi_loss = r[0]; out->baseline_loss = r[3]; out->entropy = r[4];
-    out->learning_rate = o.learning_rate; out->grad_norm = o.grad_norm; out->step = o.step;
+    out->learning_rate = r[1]; out->grad_norm = r[2]; out->step = result_row_step(r);
   }
   return DRL_OK;
 }
@@ -1368,11 +864,9 @@ int drl_a3c_step(drl_a3c* h, int32_t slot, drl_a3c_out* out) {
   return drl_a3c_wait(h, out);
 }
 int drl_a3c_act(drl_a3c* h, int32_t n, const uint8_t* state, const int32_t* previous_action, float* policy, float* value) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
+  DRL_ENTER(h);
   if (n < 1 || n > 2 * h->B) { set_error("act: n must be in [1, %d]", 2 * h->B); return DRL_ERR_INVALID; }
   if (!state || !previous_action) { set_error("act: null pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   ApexSlot& s = h->slots[h->cfg.num_slots];
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
   DRL_TRY(stage_into(h, s, h->compute, n, n, state, nullptr, previous_action, nullptr, nullptr, nullptr, nullptr));
@@ -1383,16 +877,14 @@ int drl_a3c_act(drl_a3c* h, int32_t n, const uint8_t* state, const int32_t* prev
   if (policy) DRL_CUDA_CHECK(cudaMemcpyAsync(policy, h->act.scratch_sm, (size_t)n * h->A * 4, cudaMemcpyDeviceToHost, h->compute));
   if (value) DRL_CUDA_CHECK(cudaMemcpyAsync(value, h->act.mstream, (size_t)n * 4, cudaMemcpyDeviceToHost, h->compute));
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  h->last_n = 0;
+  h->last_rows = 0;
   return DRL_OK;
 }
 int drl_a3c_taps(drl_a3c* h, float* policy, float* value, float* next_value, float* advantage) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_apex*>(h)->mu);
-  DRL_TRY(set_device(h));
-  if (h->last_n < 1) { set_error("taps: no step has run"); return DRL_ERR_STATE; }
+  DRL_ENTER(h);
+  if (h->last_rows < 1) { set_error("taps: no step has run"); return DRL_ERR_STATE; }
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  const size_t n = h->last_n, A = h->A;
+  const size_t n = h->last_rows, A = h->A;
   if (policy) DRL_CUDA_CHECK(cudaMemcpy(policy, h->act.scratch_sm, n * A * 4, cudaMemcpyDeviceToHost));
   if (value) DRL_CUDA_CHECK(cudaMemcpy(value, h->act.mstream, n * 4, cudaMemcpyDeviceToHost));
   if (next_value) DRL_CUDA_CHECK(cudaMemcpy(next_value, h->act.mstream + n, n * 4, cudaMemcpyDeviceToHost));

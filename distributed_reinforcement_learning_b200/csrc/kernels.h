@@ -1,6 +1,11 @@
 // kernels.h -- internal interface between the learner orchestration (learner.cu) and the kernel
 // launchers (layers.cu, elementwise.cu, vtrace.cu, optimizer.cu).  Not part of the C-ABI.
 #pragma once
+#include <string.h>
+
+#include <mutex>
+#include <vector>
+
 #include "common.cuh"
 
 namespace drl {
@@ -10,17 +15,37 @@ namespace drl {
 // kernel (kernel sizes are multiples of 4) and is padded up to a multiple of 4 floats so that all
 // kernels start 16-byte aligned.  [w ; b] therefore forms one contiguous [(K+1), N] matrix, which
 // is what the weight-gradient GEMMs write (bias gradient = column sum of dY in row K).
-struct ParamLayout {
+// The IMPALA, Ape-X and R2D2 layouts extend this with their named offsets.
+template <int N>
+struct FlatLayout {
+  static constexpr int kNumTensors = N;
+  int64_t padded_total;   // floats in the padded vector (multiple of 4)
+  int64_t packed_total;   // floats in the TF-flat (API) vector
+  int64_t packed_off[N], padded_off[N], count[N];
+  // tensor i has sizes[i] floats; *fields[i] receives its padded offset
+  void place(const int64_t (&sizes)[N], int64_t* const (&fields)[N]) {
+    int64_t po = 0, pk = 0;
+    for (int i = 0; i < N; ++i) {
+      count[i] = sizes[i];
+      packed_off[i] = pk;
+      padded_off[i] = po;
+      *fields[i] = po;
+      pk += sizes[i];
+      po += sizes[i];
+      if (i & 1) po = (po + 3) / 4 * 4;   // pad after each bias (all kernel sizes are multiples of 4)
+    }
+    packed_total = pk;
+    padded_total = (po + 3) / 4 * 4;
+  }
+};
+
+struct ParamLayout : FlatLayout<24> {
   int A;
   int64_t conv1_w, conv1_b, conv2_w, conv2_b, conv3_w, conv3_b;
   int64_t emb1_w, emb1_b, emb2_w, emb2_b;
   int64_t lstm_w, lstm_b;
   int64_t actor1_w, actor1_b, actor2_w, actor2_b, actor3_w, actor3_b;
   int64_t critic1_w, critic1_b, critic2_w, critic2_b, critic3_w, critic3_b;
-  int64_t padded_total;   // floats in the padded vector (multiple of 4)
-  int64_t packed_total;   // floats in the TF-flat (API) vector
-  static constexpr int kNumTensors = 24;
-  int64_t packed_off[kNumTensors], padded_off[kNumTensors], count[kNumTensors];
   void init(int num_action);
 };
 
@@ -193,7 +218,7 @@ struct OptState {
 int optimizer_apply(cudaStream_t s, const OptState& o);
 int optimizer_update_only(cudaStream_t s, const OptState& o);   // clip + RMSProp from already reduced partials
 
-// ---- apex.cu: TF1 Adam (shared by the Ape-X and the R2D2 learner) -------------------------------------------------
+// TF1 Adam (the Ape-X, A3C and R2D2 learners)
 // clip_norm <= 0: no clipping (optimizer.minimize, agent/r2d2.py:92); start_lr == end_lr: constant learning rate
 struct AdamState {
   float* params; float* m; float* v; const float* grads; int64_t n;
@@ -206,6 +231,7 @@ struct AdamState {
                             // (1 for a single replica); applied to the gradient, its norm and the logged losses
 };
 int adam_step(cudaStream_t s, const AdamState& o);   // 2 launches: partial norms + scalars, then the update
+constexpr float kAdamBeta1 = 0.9f, kAdamBeta2 = 0.999f;
 
 // ---- peer.cu: gradient exchange over NVLink peer memory (CUDA IPC), fused with the norm ------------------------
 constexpr int kMaxPeers = 16;
@@ -229,5 +255,85 @@ struct PeerPlan {
 };
 // one exchange instance over float4 range [beg4, end4) of the bucket; do_lr: also lr / global_step (last instance)
 int peer_exchange(cudaStream_t s, const PeerPlan& pp, int part, int64_t beg4, int64_t end4, bool do_lr, int grid = 0);
+
+// ---- host-side handle helpers (learner.cu, apex.cu, r2d2.cu) ----------------------------------------------------
+// Prologue of every C-ABI entry point that takes a handle: null check, the handle's recursive lock (actor threads call
+// parameter_sync -> get_params on the learner's handle while the learner thread trains; ctypes drops the GIL), and
+// the handle's device.
+#define DRL_ENTER(h)                                                                  \
+  if (!(h)) { ::drl::set_error("null handle"); return DRL_ERR_INVALID; }             \
+  std::lock_guard<std::recursive_mutex> _drl_lock((h)->mu);                           \
+  DRL_CUDA_CHECK(cudaSetDevice((h)->cfg.device))
+
+// zeroed (or fill_byte) device buffer of count T plus 256 bytes of slack, freed with the handle (h->allocs)
+template <class H, class T>
+int dev_alloc(H* h, T** p, size_t count, int fill_byte = 0) {
+  void* q = nullptr;
+  DRL_CUDA_CHECK(cudaMalloc(&q, count * sizeof(T) + 256));
+  DRL_CUDA_CHECK(cudaMemset(q, fill_byte, count * sizeof(T) + 256));
+  h->allocs.push_back(q);
+  *p = static_cast<T*>(q);
+  return DRL_OK;
+}
+inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// packed (TF-flat, API) <-> padded (device) copies on stream s through the pinned scratch h_flat (padded_total floats)
+template <class L>
+int upload_flat(const L& pl, float* h_flat, cudaStream_t s, float* dev_padded, const float* host_packed,
+                float pad_value = 0.0f) {
+  for (int64_t i = 0; i < pl.padded_total; ++i) h_flat[i] = pad_value;
+  for (int i = 0; i < L::kNumTensors; ++i)
+    memcpy(h_flat + pl.padded_off[i], host_packed + pl.packed_off[i], pl.count[i] * sizeof(float));
+  DRL_CUDA_CHECK(cudaStreamSynchronize(s));
+  DRL_CUDA_CHECK(cudaMemcpyAsync(dev_padded, h_flat, pl.padded_total * sizeof(float), cudaMemcpyHostToDevice, s));
+  DRL_CUDA_CHECK(cudaStreamSynchronize(s));
+  return DRL_OK;
+}
+template <class L>
+int download_flat(const L& pl, float* h_flat, cudaStream_t s, const float* dev_padded, float* host_packed) {
+  DRL_CUDA_CHECK(cudaMemcpyAsync(h_flat, dev_padded, pl.padded_total * sizeof(float), cudaMemcpyDeviceToHost, s));
+  DRL_CUDA_CHECK(cudaStreamSynchronize(s));
+  for (int i = 0; i < L::kNumTensors; ++i)
+    memcpy(host_packed + pl.packed_off[i], h_flat + pl.padded_off[i], pl.count[i] * sizeof(float));
+  return DRL_OK;
+}
+
+// captures what enqueue() puts on stream s (and the streams it forks to) and instantiates it into *exec
+template <class F>
+int capture_graph(cudaStream_t s, cudaGraphExec_t* exec, F&& enqueue) {
+  cudaGraph_t g = nullptr;
+  DRL_CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+  const int r = enqueue();
+  const cudaError_t e = cudaStreamEndCapture(s, &g);
+  if (r != DRL_OK) { if (g) cudaGraphDestroy(g); return r; }
+  if (e != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(e)); return DRL_ERR_CUDA; }
+  DRL_CUDA_CHECK(cudaGraphInstantiate(exec, g, 0));
+  cudaGraphDestroy(g);
+  return DRL_OK;
+}
+
+// read_buffer: copies the named device buffer of tab[0, n) to host_dst once compute has drained
+struct NamedBuffer { const char* name; const float* p; size_t count; };
+inline int read_named_buffer(cudaStream_t compute, const NamedBuffer* tab, size_t n, const char* name, float* host_dst,
+                             int64_t count) {
+  for (size_t i = 0; i < n; ++i) {
+    const NamedBuffer& e = tab[i];
+    if (strcmp(e.name, name) != 0) continue;
+    if ((size_t)count != e.count) { set_error("read_buffer(%s): expected %zu floats, got %lld", name, e.count, (long long)count); return DRL_ERR_INVALID; }
+    DRL_CUDA_CHECK(cudaStreamSynchronize(compute));
+    DRL_CUDA_CHECK(cudaMemcpy(host_dst, e.p, e.count * sizeof(float), cudaMemcpyDeviceToHost));
+    return DRL_OK;
+  }
+  set_error("read_buffer: unknown buffer '%s'", name);
+  return DRL_ERR_INVALID;
+}
+
+// global_step of a result row: the update kernel stores it as two int32 bit patterns in r[6] (low) and r[7] (high)
+inline int64_t result_row_step(const float* r) {
+  uint32_t lo, hi;
+  memcpy(&lo, &r[6], 4);
+  memcpy(&hi, &r[7], 4);
+  return (int64_t)(((uint64_t)hi << 32) | lo);
+}
 
 }  // namespace drl

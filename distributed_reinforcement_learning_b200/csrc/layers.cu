@@ -12,28 +12,14 @@ namespace drl {
 
 void ParamLayout::init(int num_action) {
   A = num_action;
-  const int64_t sizes[kNumTensors] = {
-      8 * 8 * 4 * 32, 32, 4 * 4 * 32 * 64, 64, 3 * 3 * 64 * 64, 64,
-      (int64_t)A * 256, 256, 256 * 256, 256,
-      (int64_t)Geo::XK * Geo::G4, Geo::G4,
-      256 * 256, 256, 256 * 256, 256, 256 * (int64_t)A, A,
-      256 * 256, 256, 256 * 256, 256, 256, 1};
-  int64_t po = 0, pk = 0;
-  for (int i = 0; i < kNumTensors; ++i) {
-    count[i] = sizes[i];
-    packed_off[i] = pk;
-    padded_off[i] = po;
-    pk += sizes[i];
-    po += sizes[i];
-    if (i & 1) po = (po + 3) / 4 * 4;   // pad after each bias (all kernel sizes are multiples of 4)
-  }
-  packed_total = pk;
-  padded_total = (po + 3) / 4 * 4;
-  int64_t* f[kNumTensors] = {&conv1_w, &conv1_b, &conv2_w, &conv2_b, &conv3_w, &conv3_b, &emb1_w, &emb1_b,
-                             &emb2_w, &emb2_b, &lstm_w, &lstm_b, &actor1_w, &actor1_b, &actor2_w, &actor2_b,
-                             &actor3_w, &actor3_b, &critic1_w, &critic1_b, &critic2_w, &critic2_b, &critic3_w,
-                             &critic3_b};
-  for (int i = 0; i < kNumTensors; ++i) *f[i] = padded_off[i];
+  place({8 * 8 * 4 * 32, 32, 4 * 4 * 32 * 64, 64, 3 * 3 * 64 * 64, 64,
+         (int64_t)A * 256, 256, 256 * 256, 256,
+         (int64_t)Geo::XK * Geo::G4, Geo::G4,
+         256 * 256, 256, 256 * 256, 256, 256 * (int64_t)A, A,
+         256 * 256, 256, 256 * 256, 256, 256, 1},
+        {&conv1_w, &conv1_b, &conv2_w, &conv2_b, &conv3_w, &conv3_b, &emb1_w, &emb1_b, &emb2_w, &emb2_b, &lstm_w,
+         &lstm_b, &actor1_w, &actor1_b, &actor2_w, &actor2_b, &actor3_w, &actor3_b, &critic1_w, &critic1_b, &critic2_w,
+         &critic2_b, &critic3_w, &critic3_b});
 }
 
 static int g_fwd_launches = 0, g_bwd_launches = 0;

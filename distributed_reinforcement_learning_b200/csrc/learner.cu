@@ -169,58 +169,17 @@ struct drl_learner {
   // reference's launchers nevertheless has actor threads call parameter_sync() -> get_params on the learner's handle
   // while the learner thread trains, and ctypes drops the GIL.  Every entry point therefore takes this lock (the
   // pinned staging buffer h_flat, `pending`, `last_out` and the graph caches are all guarded by it).
-  std::recursive_mutex mu;
+  mutable std::recursive_mutex mu;
 };
-#define DRL_LOCK(h) std::lock_guard<std::recursive_mutex> _drl_lock((h)->mu)
 
 namespace {
 
-template <class T>
-int dev_alloc(drl_learner* h, T** p, size_t count, int fill_byte = 0) {
-  void* q = nullptr;
-  DRL_CUDA_CHECK(cudaMalloc(&q, count * sizeof(T) + 256));
-  DRL_CUDA_CHECK(cudaMemset(q, fill_byte, count * sizeof(T) + 256));
-  h->allocs.push_back(q);
-  *p = static_cast<T*>(q);
-  return DRL_OK;
-}
-
-size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-int check_handle(const drl_learner* h) {
-  if (!h) { set_error("null learner handle"); return DRL_ERR_INVALID; }
-  return DRL_OK;
-}
 int check_not_failed(const drl_learner* h) {
   if (h->failed) {
     set_error("learner handle is in the failed state (a peer-exchange barrier timed out): parameters and optimizer "
               "state are not readable and no further step can run");
     return DRL_ERR_STATE;
   }
-  return DRL_OK;
-}
-
-int set_device(const drl_learner* h) {
-  DRL_CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  return DRL_OK;
-}
-
-// packed (TF-flat, API) <-> padded (device) copies through the pinned scratch
-int upload_flat(drl_learner* h, float* dev_padded, const float* host_packed, float pad_value) {
-  for (int64_t i = 0; i < h->pl.padded_total; ++i) h->h_flat[i] = pad_value;
-  for (int i = 0; i < ParamLayout::kNumTensors; ++i)
-    memcpy(h->h_flat + h->pl.padded_off[i], host_packed + h->pl.packed_off[i], h->pl.count[i] * sizeof(float));
-  DRL_CUDA_CHECK(cudaMemcpyAsync(dev_padded, h->h_flat, h->pl.padded_total * sizeof(float), cudaMemcpyHostToDevice,
-                                 h->compute));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  return DRL_OK;
-}
-int download_flat(drl_learner* h, const float* dev_padded, float* host_packed) {
-  DRL_CUDA_CHECK(cudaMemcpyAsync(h->h_flat, dev_padded, h->pl.padded_total * sizeof(float), cudaMemcpyDeviceToHost,
-                                 h->compute));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  for (int i = 0; i < ParamLayout::kNumTensors; ++i)
-    memcpy(host_packed + h->pl.packed_off[i], h->h_flat + h->pl.padded_off[i], h->pl.count[i] * sizeof(float));
   return DRL_OK;
 }
 
@@ -311,14 +270,7 @@ int run_forward_backward(drl_learner* h, int slot) {
       // one eager pass first: sets the per-kernel shared-memory attributes outside of stream capture
       // (idempotent: every buffer it writes is fully overwritten by the captured pass)
       DRL_TRY(enqueue_forward_backward(h, slot));
-      cudaGraph_t g = nullptr;
-      DRL_CUDA_CHECK(cudaStreamBeginCapture(h->compute, cudaStreamCaptureModeThreadLocal));
-      int r = enqueue_forward_backward(h, slot);
-      cudaError_t e = cudaStreamEndCapture(h->compute, &g);
-      if (r != DRL_OK) { if (g) cudaGraphDestroy(g); return r; }
-      if (e != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(e)); return DRL_ERR_CUDA; }
-      DRL_CUDA_CHECK(cudaGraphInstantiate(&h->graph_fb[slot], g, 0));
-      cudaGraphDestroy(g);
+      DRL_TRY(capture_graph(h->compute, &h->graph_fb[slot], [&] { return enqueue_forward_backward(h, slot); }));
     }
     DRL_CUDA_CHECK(cudaGraphLaunch(h->graph_fb[slot], h->compute));
   } else {
@@ -331,14 +283,7 @@ int run_forward_backward(drl_learner* h, int slot) {
 int run_apply(drl_learner* h) {
   if (h->cfg.use_cuda_graph) {
     if (!h->graph_apply) {
-      cudaGraph_t g = nullptr;
-      DRL_CUDA_CHECK(cudaStreamBeginCapture(h->compute, cudaStreamCaptureModeThreadLocal));
-      int r = enqueue_apply(h, (int)h->slots.size());
-      cudaError_t e = cudaStreamEndCapture(h->compute, &g);
-      if (r != DRL_OK) { if (g) cudaGraphDestroy(g); return r; }
-      if (e != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(e)); return DRL_ERR_CUDA; }
-      DRL_CUDA_CHECK(cudaGraphInstantiate(&h->graph_apply, g, 0));
-      cudaGraphDestroy(g);
+      DRL_TRY(capture_graph(h->compute, &h->graph_apply, [&] { return enqueue_apply(h, (int)h->slots.size()); }));
     }
     DRL_CUDA_CHECK(cudaGraphLaunch(h->graph_apply, h->compute));
   } else {
@@ -363,15 +308,10 @@ int run_step(drl_learner* h, int slot) {
   if (h->cfg.use_cuda_graph) {
     if (!h->graph_step[slot]) {
       DRL_TRY(enqueue_forward_backward(h, slot));   // eager pass: per-kernel attributes are set outside of capture
-      cudaGraph_t g = nullptr;
-      DRL_CUDA_CHECK(cudaStreamBeginCapture(h->compute, cudaStreamCaptureModeThreadLocal));
-      int r = enqueue_forward_backward(h, slot);
-      if (r == DRL_OK) r = enqueue_apply(h, slot, false, h->peer_on && h->par && h->peer_early_ctas > 0);
-      cudaError_t e = cudaStreamEndCapture(h->compute, &g);
-      if (r != DRL_OK) { if (g) cudaGraphDestroy(g); return r; }
-      if (e != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(e)); return DRL_ERR_CUDA; }
-      DRL_CUDA_CHECK(cudaGraphInstantiate(&h->graph_step[slot], g, 0));
-      cudaGraphDestroy(g);
+      DRL_TRY(capture_graph(h->compute, &h->graph_step[slot], [&] {
+        const int r = enqueue_forward_backward(h, slot);
+        return r != DRL_OK ? r : enqueue_apply(h, slot, false, h->peer_on && h->par && h->peer_early_ctas > 0);
+      }));
     }
     NvtxRange r("drl:step(graph)");
     DRL_CUDA_CHECK(cudaGraphLaunch(h->graph_step[slot], h->compute));
@@ -443,7 +383,7 @@ int drl_learner_create(const drl_learner_config* cfg, drl_learner** out) {
   h->M = h->B * h->T; h->Mb = h->B * (h->T - 2);
   h->pl.init(h->A);
   int rc = [&]() -> int {
-    DRL_TRY(set_device(h));
+    DRL_CUDA_CHECK(cudaSetDevice(h->cfg.device));
     DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->compute, cudaStreamNonBlocking));
     DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->copy, cudaStreamNonBlocking));
     DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking));
@@ -622,47 +562,38 @@ int drl_learner_destroy(drl_learner* h) {
 }
 
 int drl_learner_param_count(const drl_learner* h, int64_t* n) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!n) { set_error("null argument"); return DRL_ERR_INVALID; }
   *n = h->pl.packed_total;
   return DRL_OK;
 }
 
 int drl_learner_set_params(drl_learner* h, const float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!host_flat || n != h->pl.packed_total) { set_error("set_params: expected %lld floats, got %lld", (long long)h->pl.packed_total, (long long)n); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_TRY(upload_flat(h, h->params, host_flat, 0.0f));
+  DRL_TRY(upload_flat(h->pl, h->h_flat, h->compute, h->params, host_flat));
   h->images_stale = true;
   return DRL_OK;
 }
 int drl_learner_get_params(drl_learner* h, float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   DRL_TRY(check_not_failed(h));
   if (!host_flat || n != h->pl.packed_total) { set_error("get_params: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return download_flat(h, h->params, host_flat);
+  return download_flat(h->pl, h->h_flat, h->compute, h->params, host_flat);
 }
 int drl_learner_set_opt_state(drl_learner* h, const float* host_ms_flat, int64_t n, int64_t step) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!host_ms_flat || n != h->pl.packed_total) { set_error("set_opt_state: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_TRY(upload_flat(h, h->ms, host_ms_flat, 1.0f));
+  DRL_TRY(upload_flat(h->pl, h->h_flat, h->compute, h->ms, host_ms_flat, 1.0f));
   long long st = step;
   DRL_CUDA_CHECK(cudaMemcpy(h->d_step, &st, sizeof(st), cudaMemcpyHostToDevice));
   return DRL_OK;
 }
 int drl_learner_get_opt_state(drl_learner* h, float* host_ms_flat, int64_t n, int64_t* step) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   DRL_TRY(check_not_failed(h));
   if (n != h->pl.packed_total) { set_error("get_opt_state: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  if (host_ms_flat) DRL_TRY(download_flat(h, h->ms, host_ms_flat));
+  if (host_ms_flat) DRL_TRY(download_flat(h->pl, h->h_flat, h->compute, h->ms, host_ms_flat));
   if (step) {
     long long st = 0;
     DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
@@ -672,25 +603,21 @@ int drl_learner_get_opt_state(drl_learner* h, float* host_ms_flat, int64_t n, in
   return DRL_OK;
 }
 int drl_learner_get_grads(drl_learner* h, float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   DRL_TRY(check_not_failed(h));
   if (!host_flat || n != h->pl.packed_total) { set_error("get_grads: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return download_flat(h, h->peer_on ? reinterpret_cast<float*>(h->comm) : h->bucket, host_flat);
+  return download_flat(h->pl, h->h_flat, h->compute, h->peer_on ? reinterpret_cast<float*>(h->comm) : h->bucket, host_flat);
 }
 
 int drl_learner_stage(drl_learner* h, int32_t slot, const uint8_t* state, const float* reward, const int32_t* action,
                       const uint8_t* done, const float* behavior_policy, const int32_t* previous_action,
                       const float* initial_h, const float* initial_c) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (slot < 0 || slot >= (int)h->slots.size()) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
   if (!state || !reward || !action || !done || !behavior_policy || !previous_action || !initial_h || !initial_c) {
     set_error("stage: null input pointer");
     return DRL_ERR_INVALID;
   }
-  DRL_TRY(set_device(h));
   NvtxRange nvtx_r("drl:stage");
   Slot& s = h->slots[slot];
   const size_t BT = (size_t)h->B * h->T;
@@ -713,44 +640,36 @@ int drl_learner_stage(drl_learner* h, int32_t slot, const uint8_t* state, const 
 }
 
 int drl_learner_forward_backward(drl_learner* h, int32_t slot) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   DRL_TRY(check_not_failed(h));
   if (slot < 0 || slot >= (int)h->slots.size()) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   return run_forward_backward(h, slot);
 }
 
 int drl_learner_grad_bucket(drl_learner* h, void** dev_ptr, int64_t* count) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (dev_ptr) *dev_ptr = h->bucket;
   if (count) *count = h->pl.padded_total + 4;
   return DRL_OK;
 }
 
 int drl_learner_reduced_bucket(drl_learner* h, void** dev_ptr, int64_t* count) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(h);
+  DRL_ENTER(h);
   if (dev_ptr) *dev_ptr = h->peer_on ? static_cast<void*>(h->comm) : static_cast<void*>(h->bucket);
   if (count) *count = h->pl.padded_total + 4;
   return DRL_OK;
 }
 
 int drl_learner_apply(drl_learner* h) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   DRL_TRY(check_not_failed(h));
-  DRL_TRY(set_device(h));
   return run_apply(h);
 }
 
 // ---- gradient exchange over NVLink peer memory (peer.cu) -------------------------------------------------------
 int drl_learner_peer_export(drl_learner* h, void* handles, int64_t bytes) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!handles || bytes != 2 * (int64_t)sizeof(cudaIpcMemHandle_t)) { set_error("peer_export: expected a %d-byte buffer", (int)(2 * sizeof(cudaIpcMemHandle_t))); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   if (!h->comm) {
     const size_t red = align_up((size_t)(h->pl.padded_total + 4) * sizeof(float), 256);
     h->off_partials = red;
@@ -771,13 +690,11 @@ int drl_learner_peer_export(drl_learner* h, void* handles, int64_t bytes) {
 }
 
 int drl_learner_peer_import(drl_learner* h, int32_t rank, int32_t world, const void* all_handles, int64_t bytes) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (world < 2 || world > kMaxPeers || rank < 0 || rank >= world) { set_error("peer_import: bad rank %d / world %d (max %d)", rank, world, kMaxPeers); return DRL_ERR_INVALID; }
   if (!all_handles || bytes != (int64_t)world * 2 * (int64_t)sizeof(cudaIpcMemHandle_t)) { set_error("peer_import: expected world x %d bytes", (int)(2 * sizeof(cudaIpcMemHandle_t))); return DRL_ERR_INVALID; }
   if (!h->comm) { set_error("peer_import before peer_export"); return DRL_ERR_STATE; }
   if (h->peer_on) { set_error("peer exchange already set up"); return DRL_ERR_STATE; }
-  DRL_TRY(set_device(h));
   DRL_CUDA_CHECK(cudaDeviceSynchronize());
   const cudaIpcMemHandle_t* hd = static_cast<const cudaIpcMemHandle_t*>(all_handles);
   for (int p = 0; p < world; ++p) {
@@ -830,9 +747,7 @@ int drl_learner_peer_import(drl_learner* h, int32_t rank, int32_t world, const v
 }
 
 int drl_learner_peer_disable(drl_learner* h) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
-  DRL_TRY(set_device(h));
+  DRL_ENTER(h);
   DRL_CUDA_CHECK(cudaDeviceSynchronize());
   for (void* p : h->peer_opened) cudaIpcCloseMemHandle(p);
   h->peer_opened.clear();
@@ -846,19 +761,16 @@ int drl_learner_peer_disable(drl_learner* h) {
 }
 
 int drl_learner_stream(drl_learner* h, void** stream) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!stream) { set_error("null argument"); return DRL_ERR_INVALID; }
   *stream = h->compute;
   return DRL_OK;
 }
 
 int drl_learner_step_async(drl_learner* h, int32_t slot) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   DRL_TRY(check_not_failed(h));
   if (slot < 0 || slot >= (int)h->slots.size()) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   return run_step(h, slot);
 }
 
@@ -879,44 +791,34 @@ static int collect(drl_learner* h, int row, drl_step_out* out) {
     out->learning_rate = r[3];
     out->grad_norm = r[4];
     out->total_loss = r[5];
-    uint32_t lo, hi;
-    memcpy(&lo, &r[6], 4);
-    memcpy(&hi, &r[7], 4);
-    out->step = (int64_t)(((uint64_t)hi << 32) | lo);
+    out->step = result_row_step(r);
   }
   return DRL_OK;
 }
 
 int drl_learner_wait(drl_learner* h, drl_step_out* out) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!h->pending) { set_error("wait: no step in flight"); return DRL_ERR_STATE; }
-  DRL_TRY(set_device(h));
   h->pending = false;
   return collect(h, h->last_out, out);
 }
 
 int drl_learner_wait_slot(drl_learner* h, int32_t slot, drl_step_out* out) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (slot < 0 || slot >= (int)h->slots.size()) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   if (slot == h->last_out) h->pending = false;
   return collect(h, slot, out);
 }
 
 int drl_learner_step(drl_learner* h, int32_t slot, drl_step_out* out) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(h);
+  DRL_ENTER(h);
   DRL_TRY(drl_learner_step_async(h, slot));
   return drl_learner_wait(h, out);
 }
 
 int drl_learner_forward(drl_learner* h, int32_t slot, float* policy, float* value) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (slot < 0 || slot >= (int)h->slots.size()) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   Slot& s = h->slots[slot];
   if (!s.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
   DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, s.staged, 0));
@@ -939,9 +841,7 @@ int drl_learner_forward(drl_learner* h, int32_t slot, float* policy, float* valu
 }
 
 int drl_learner_taps(drl_learner* h, float* vs, float* clipped_rho, float* vs_plus_1, float* pg_advantage) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
-  DRL_TRY(set_device(h));
+  DRL_ENTER(h);
   const size_t n = (size_t)h->B * (h->T - 2) * sizeof(float);
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
   if (vs) DRL_CUDA_CHECK(cudaMemcpy(vs, h->vt.vs, n, cudaMemcpyDeviceToHost));
@@ -952,13 +852,10 @@ int drl_learner_taps(drl_learner* h, float* vs, float* clipped_rho, float* vs_pl
 }
 
 int drl_learner_read_buffer(drl_learner* h, const char* name, float* host_dst, int64_t n) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!name || !host_dst) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   const size_t M = h->M, Mb = h->Mb, A = h->A;
-  struct Ent { const char* nm; const float* p; size_t cnt; };
-  const Ent tab[] = {
+  const NamedBuffer tab[] = {
       {"a1", h->act.a1, M * 400 * 32}, {"a2", h->act.a2, M * 81 * 64}, {"a3", h->act.a3, M * Geo::FLAT},
       {"emb", h->act.table, A * Geo::EMB}, {"e1", h->act.e1, A * Geo::EMB},
       {"gates", h->act.gates, M * Geo::G4}, {"h1", h->act.h1, M * Geo::L}, {"c1", h->act.c1, M * Geo::L},
@@ -968,25 +865,14 @@ int drl_learner_read_buffer(drl_learner* h, const char* name, float* host_dst, i
       {"dhid1", h->bwd.dhid1, 2 * Mb * Geo::HID}, {"dh_part", h->bwd.dh_part, 2 * Mb * Geo::L},
       {"dz", h->bwd.dz, Mb * Geo::G4}, {"da3", h->bwd.da3, Mb * Geo::FLAT}, {"du", h->bwd.du, Mb * Geo::EMB},
       {"da2", h->bwd.da2, Mb * 81 * 64}, {"da1", h->bwd.da1, Mb * 400 * 32}};
-  for (const Ent& e : tab) {
-    if (strcmp(e.nm, name) == 0) {
-      if ((size_t)n != e.cnt) { set_error("read_buffer(%s): expected %zu floats, got %lld", name, e.cnt, (long long)n); return DRL_ERR_INVALID; }
-      DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-      DRL_CUDA_CHECK(cudaMemcpy(host_dst, e.p, e.cnt * sizeof(float), cudaMemcpyDeviceToHost));
-      return DRL_OK;
-    }
-  }
-  set_error("read_buffer: unknown buffer '%s'", name);
-  return DRL_ERR_INVALID;
+  return read_named_buffer(h->compute, tab, sizeof(tab) / sizeof(tab[0]), name, host_dst, n);
 }
 
 int drl_learner_act(drl_learner* h, int32_t n, const uint8_t* state, const int32_t* previous_action,
                     const float* h_in, const float* c_in, float* policy, float* h_out, float* c_out) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (n < 1 || n > h->M) { set_error("act: n must be in [1, %d]", h->M); return DRL_ERR_INVALID; }
   if (!state || !previous_action || !h_in || !c_in) { set_error("act: null input pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   // reuse staging slot 0 as an [n, 1] batch (B = n, T = 1 makes the time-major/batch-major remap the identity)
   Slot& s = h->slots[0];
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
@@ -1010,11 +896,9 @@ int drl_learner_act(drl_learner* h, int32_t n, const uint8_t* state, const int32
 
 int drl_learner_profile_step(drl_learner* h, int32_t slot, char* names, int64_t names_len, float* ms,
                              int32_t max_kernels, int32_t* count) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (slot < 0 || slot >= (int)h->slots.size()) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
   if (!names || !ms || !count) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   Slot& sl = h->slots[slot];
   if (!sl.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
   DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, sl.staged, 0));
@@ -1031,18 +915,15 @@ int drl_learner_profile_step(drl_learner* h, int32_t slot, char* names, int64_t 
 }
 
 int drl_learner_last_step_ms(drl_learner* h, float* ms) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!ms) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
   DRL_CUDA_CHECK(cudaEventSynchronize(h->ev_stop));
   DRL_CUDA_CHECK(cudaEventElapsedTime(ms, h->ev_start, h->ev_stop));
   return DRL_OK;
 }
 
 int drl_learner_launches_per_step(const drl_learner* h, int32_t* n) {
-  DRL_TRY(check_handle(h));
-  DRL_LOCK(const_cast<drl_learner*>(h));
+  DRL_ENTER(h);
   if (!n) { set_error("null argument"); return DRL_ERR_INVALID; }
   // forward + V-trace/loss kernel + backward + 2 optimizer kernels (valid after the first step)
   *n = forward_launch_count() + 1 + backward_launch_count() + 2;

@@ -10,13 +10,7 @@
 // persistent CTA per sequence keeps W_h in shared memory and walks the S steps (r2d2_lstm_fwd_kernel); BPTT is the
 // mirror image (r2d2_lstm_bwd_kernel, W_h^T in shared memory), after which every weight / data gradient is again one
 // batched GEMM over all M rows (all rows receive gradient: burn-in only slices the loss, agent/r2d2.py:64-68).
-#include <string.h>
-
-#include <string>
-#include <mutex>
-#include <vector>
-
-#include "layer_defs.cuh"
+#include "adam_learner.cuh"
 
 namespace drl {
 
@@ -25,34 +19,18 @@ constexpr int kR2G = 4 * kR2L;           // 256 gate columns
 constexpr int kR2H = 128;                // dense width between the LSTM and the two output streams (model/r2d2_lstm.py:50)
 constexpr int kR2Cat = Geo::FLAT + Geo::EMB;   // 3392 rows of the LSTM kernel that multiply the step input
 
-struct R2Layout {
+struct R2Layout : FlatLayout<18> {
   int A, C;
   int64_t conv1_w, conv1_b, conv2_w, conv2_b, conv3_w, conv3_b, emb1_w, emb1_b, emb2_w, emb2_b;
   int64_t lstm_w, lstm_b, q1_w, q1_b, value_w, value_b, mean_w, mean_b;
-  int64_t padded_total, packed_total;
-  static constexpr int kNumTensors = 18;
-  int64_t packed_off[kNumTensors], padded_off[kNumTensors], count[kNumTensors];
   void init(int num_action, int channels) {
     A = num_action; C = channels;
-    const int64_t sizes[kNumTensors] = {
-        8 * 8 * (int64_t)C * 32, 32, 4 * 4 * 32 * 64, 64, 3 * 3 * 64 * 64, 64,
-        (int64_t)A * 256, 256, 256 * 256, 256,
-        (int64_t)(kR2Cat + kR2L) * kR2G, kR2G,
-        (int64_t)kR2L * kR2H, kR2H, (int64_t)kR2H * A, A, kR2H, 1};
-    int64_t po = 0, pk = 0;
-    for (int i = 0; i < kNumTensors; ++i) {
-      count[i] = sizes[i];
-      packed_off[i] = pk;
-      padded_off[i] = po;
-      pk += sizes[i];
-      po += sizes[i];
-      if (i & 1) po = (po + 3) / 4 * 4;
-    }
-    packed_total = pk;
-    padded_total = (po + 3) / 4 * 4;
-    int64_t* f[kNumTensors] = {&conv1_w, &conv1_b, &conv2_w, &conv2_b, &conv3_w, &conv3_b, &emb1_w, &emb1_b, &emb2_w,
-                               &emb2_b, &lstm_w, &lstm_b, &q1_w, &q1_b, &value_w, &value_b, &mean_w, &mean_b};
-    for (int i = 0; i < kNumTensors; ++i) *f[i] = padded_off[i];
+    place({8 * 8 * (int64_t)C * 32, 32, 4 * 4 * 32 * 64, 64, 3 * 3 * 64 * 64, 64,
+           (int64_t)A * 256, 256, 256 * 256, 256,
+           (int64_t)(kR2Cat + kR2L) * kR2G, kR2G,
+           (int64_t)kR2L * kR2H, kR2H, (int64_t)kR2H * A, A, kR2H, 1},
+          {&conv1_w, &conv1_b, &conv2_w, &conv2_b, &conv3_w, &conv3_b, &emb1_w, &emb1_b, &emb2_w, &emb2_b, &lstm_w,
+           &lstm_b, &q1_w, &q1_b, &value_w, &value_b, &mean_w, &mean_b});
   }
 };
 
@@ -639,103 +617,22 @@ static int r2_backward(const Streams& st, const R2Layout& pl, const float* P, co
   return DRL_OK;
 }
 
-struct R2Slot {
-  uint8_t* base = nullptr;
-  R2In in{};
-  cudaEvent_t staged = nullptr, consumed = nullptr;
-  bool has_data = false;
-};
-
 }  // namespace drl
 
 using namespace drl;
 
-struct drl_r2d2 {
-  std::recursive_mutex mu;   // every C-ABI entry point locks the handle (actor threads call parameter_sync -> get_params
-                             // on the learner's handle while the learner thread trains; ctypes drops the GIL)
+struct drl_r2d2 : AdamLearner {
   drl_r2d2_config cfg{};
-  int B = 0, S = 0, A = 0, C = 1, mode = 2, Nt = 0;
+  int S = 0, A = 0, C = 1, Nt = 0;
   size_t frame = 0;
   R2Layout pl{};
-  cudaStream_t compute = nullptr, copy = nullptr, side = nullptr;
-  cudaEvent_t ev_start = nullptr, ev_stop = nullptr, ev_done = nullptr;
-  cudaEvent_t fj[8] = {};
-  // the target scope's forward is independent of the main scope's: it runs on its own stream pair beside it
-  cudaStream_t tmain = nullptr, tside = nullptr;
-  cudaEvent_t tfj[8] = {}, ev_tfork = nullptr, ev_tjoin = nullptr;
-  bool par = true;
-  float *params = nullptr, *target = nullptr, *adam_m = nullptr, *adam_v = nullptr, *grads = nullptr;
   R2Acts act{}, tact{};
   R2Bwd bwd{};
-  WeightImages wi{}, twi{};
-  bool main_images_stale = true, target_images_stale = true;
-  float *sav = nullptr, *target_value = nullptr, *td_dev = nullptr, *loss = nullptr, *c_last = nullptr;
-  int last_b = 0;
-  AdamState opt{};
-  long long* d_step = nullptr;
-  float *d_lr = nullptr, *d_alpha = nullptr, *d_b1p = nullptr, *d_b2p = nullptr;
-  float *h_out = nullptr, *d_out = nullptr, *h_td = nullptr, *d_td = nullptr, *h_flat = nullptr, *h_ones = nullptr;
-  std::vector<R2Slot> slots;            // num_slots + 1 scratch slot
-  std::vector<void*> allocs;
-  std::vector<cudaGraphExec_t> graph_step;
-  bool pending = false;
-  int last_slot = 0, launches = 0;
+  float *sav = nullptr, *target_value = nullptr, *td_dev = nullptr, *c_last = nullptr;
+  std::vector<R2In> slots;     // payloads of AdamLearner::sync
 };
 
 namespace {
-
-template <class T>
-int dev_alloc(drl_r2d2* h, T** p, size_t count) {
-  void* q = nullptr;
-  DRL_CUDA_CHECK(cudaMalloc(&q, count * sizeof(T) + 256));
-  DRL_CUDA_CHECK(cudaMemset(q, 0, count * sizeof(T) + 256));
-  h->allocs.push_back(q);
-  *p = static_cast<T*>(q);
-  return DRL_OK;
-}
-size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-int check_handle(const drl_r2d2* h) {
-  if (!h) { set_error("null r2d2 handle"); return DRL_ERR_INVALID; }
-  return DRL_OK;
-}
-int set_device(const drl_r2d2* h) {
-  DRL_CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  return DRL_OK;
-}
-int upload_flat(drl_r2d2* h, float* dev_padded, const float* host_packed) {
-  for (int64_t i = 0; i < h->pl.padded_total; ++i) h->h_flat[i] = 0.0f;
-  for (int i = 0; i < R2Layout::kNumTensors; ++i)
-    memcpy(h->h_flat + h->pl.padded_off[i], host_packed + h->pl.packed_off[i], h->pl.count[i] * sizeof(float));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  DRL_CUDA_CHECK(cudaMemcpyAsync(dev_padded, h->h_flat, h->pl.padded_total * sizeof(float), cudaMemcpyHostToDevice, h->compute));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  return DRL_OK;
-}
-int download_flat(drl_r2d2* h, const float* dev_padded, float* host_packed) {
-  DRL_CUDA_CHECK(cudaMemcpyAsync(h->h_flat, dev_padded, h->pl.padded_total * sizeof(float), cudaMemcpyDeviceToHost, h->compute));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  for (int i = 0; i < R2Layout::kNumTensors; ++i)
-    memcpy(host_packed + h->pl.packed_off[i], h->h_flat + h->pl.padded_off[i], h->pl.count[i] * sizeof(float));
-  return DRL_OK;
-}
-// stream pair of the target scope: its own pair when the step runs parallel, otherwise the main pair (serial)
-Streams target_streams_of(const drl_r2d2* h) {
-  Streams st;
-  st.main = h->par ? h->tmain : h->compute;
-  st.side = h->par ? h->tside : h->side;
-  for (int i = 0; i < 8; ++i) st.ev[i] = h->par ? h->tfj[i] : h->fj[i];
-  st.par = h->par;
-  return st;
-}
-
-Streams streams_of(const drl_r2d2* h) {
-  Streams st;
-  st.main = h->compute;
-  st.side = h->side;
-  for (int i = 0; i < 8; ++i) st.ev[i] = h->fj[i];
-  st.par = h->par;
-  return st;
-}
 
 int alloc_acts(drl_r2d2* h, R2Acts& a) {
   const size_t M = (size_t)h->B * h->S, A = h->A;
@@ -766,23 +663,15 @@ int enqueue_forward_td(drl_r2d2* h, const R2In& in, int nb, bool train, float* t
   const Streams st = streams_of(h), tst = target_streams_of(h);
   // the two unrolls are independent (and each recurrence kernel only occupies nb SMs): the target scope runs on its
   // own stream pair beside the main scope and joins before the TD kernel
-  if (h->par) {
-    DRL_CUDA_CHECK(cudaEventRecord(h->ev_tfork, h->compute));
-    DRL_CUDA_CHECK(cudaStreamWaitEvent(h->tmain, h->ev_tfork, 0));
-    pdl_break(h->tmain);
-    pdl_break(h->tside);
-  }
+  DRL_TRY(fork_target(h));
   DRL_TRY(r2_forward(tst, h->pl, h->target, h->twi, in, h->tact, nullptr, nb, h->S, h->mode, h->target_images_stale, false,
                      true, launches));
   h->target_images_stale = false;
-  if (h->par) DRL_CUDA_CHECK(cudaEventRecord(h->ev_tjoin, h->tmain));
+  DRL_TRY(target_done(h));
   DRL_TRY(r2_forward(st, h->pl, h->params, h->wi, in, h->act, nullptr, nb, h->S, h->mode, h->main_images_stale,
                      h->main_images_stale, false, launches));
   h->main_images_stale = false;
-  if (h->par) {
-    DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, h->ev_tjoin, 0));
-    pdl_break(h->compute);
-  }
+  DRL_TRY(join_target(h));
   R2TdArgs a{};
   a.mq = h->act.q; a.tq = h->tact.q;
   a.action = in.action; a.reward = in.reward; a.done = in.done; a.weight = train ? in.weight : nullptr;
@@ -796,113 +685,29 @@ int enqueue_forward_td(drl_r2d2* h, const R2In& in, int nb, bool train, float* t
   return DRL_OK;
 }
 
-int enqueue_step(drl_r2d2* h, int slot, int* launches) {
-  const R2In& in = h->slots[slot].in;
+// the step's unrolls, loss and BPTT (FwdBwd of the shell, adam_learner.cuh)
+int forward_backward(drl_r2d2* h, int slot, int* launches) {
+  const R2In& in = h->slots[slot];
   DRL_TRY(enqueue_forward_td(h, in, h->B, true, h->d_td + (size_t)slot * h->B, launches));
-  DRL_TRY(r2_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, in, h->act, h->bwd, h->B, h->S, h->mode, launches));
-  pdl_break(h->compute);
-  AdamState o = h->opt;
-  o.out = h->d_out + 8 * slot;
-  prof_mark(h->compute, "optimizer(norm+adam)");
-  DRL_TRY(adam_step(h->compute, o));
-  prof_mark(h->compute, "end");
-  if (launches) *launches += 2;
-  return DRL_OK;
-}
-
-int refresh_target_images(drl_r2d2* h) {
-  if (h->target_images_stale && h->mode >= 2) {
-    DRL_TRY((launch_retile_b<64>(h->compute, PlainB{h->target + h->pl.conv2_w, 64, 0}, 64, 512, h->twi.img[1])));
-    DRL_TRY((launch_retile_b<64>(h->compute, PlainB{h->target + h->pl.conv3_w, 64, 0}, 64, 576, h->twi.img[2])));
-  }
-  h->target_images_stale = false;
-  return DRL_OK;
-}
-
-int run_step(drl_r2d2* h, int slot) {
-  R2Slot& sl = h->slots[slot];
-  if (!sl.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, sl.staged, 0));
-  if (h->cfg.use_cuda_graph) DRL_TRY(refresh_target_images(h));     // never part of the captured step
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_start, h->compute));
-  h->main_images_stale = true;
-  if (h->cfg.use_cuda_graph) {
-    if (!h->graph_step[slot]) {
-      DRL_TRY(enqueue_forward_td(h, sl.in, h->B, true, h->d_td + (size_t)slot * h->B, nullptr));   // eager: kernel attributes
-      DRL_TRY(r2_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, sl.in, h->act, h->bwd, h->B, h->S, h->mode, nullptr));
-      h->main_images_stale = true;
-      cudaGraph_t g = nullptr;
-      int cnt = 0;
-      DRL_CUDA_CHECK(cudaStreamBeginCapture(h->compute, cudaStreamCaptureModeThreadLocal));
-      int r = enqueue_step(h, slot, &cnt);
-      cudaError_t e = cudaStreamEndCapture(h->compute, &g);
-      if (r != DRL_OK) { if (g) cudaGraphDestroy(g); return r; }
-      if (e != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(e)); return DRL_ERR_CUDA; }
-      DRL_CUDA_CHECK(cudaGraphInstantiate(&h->graph_step[slot], g, 0));
-      cudaGraphDestroy(g);
-      h->launches = cnt;
-    }
-    DRL_CUDA_CHECK(cudaGraphLaunch(h->graph_step[slot], h->compute));
-  } else {
-    int cnt = 0;
-    DRL_TRY(enqueue_step(h, slot, &cnt));
-    h->launches = cnt;
-  }
-  h->main_images_stale = true;
-  h->last_b = h->B;
-  h->last_slot = slot;
-  DRL_CUDA_CHECK(cudaEventRecord(sl.consumed, h->compute));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_stop, h->compute));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_done, h->compute));
-  h->pending = true;
-  return DRL_OK;
-}
-
-// data parallel: the step in two halves around the caller's all-reduce of the bucket (eager launches)
-int run_forward_backward(drl_r2d2* h, int slot) {
-  R2Slot& sl = h->slots[slot];
-  if (!sl.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, sl.staged, 0));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_start, h->compute));
-  h->main_images_stale = true;
-  int cnt = 0;
-  DRL_TRY(enqueue_forward_td(h, sl.in, h->B, true, h->d_td + (size_t)slot * h->B, &cnt));
-  DRL_TRY(r2_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, sl.in, h->act, h->bwd, h->B, h->S, h->mode, &cnt));
-  h->launches = cnt + 2;
-  h->last_b = h->B;
-  h->last_slot = slot;
-  DRL_CUDA_CHECK(cudaEventRecord(sl.consumed, h->compute));
-  return DRL_OK;
-}
-int run_apply(drl_r2d2* h, float grad_scale) {
-  pdl_break(h->compute);
-  AdamState o = h->opt;
-  o.out = h->d_out + 8 * h->last_slot;
-  o.grad_scale = grad_scale;
-  DRL_TRY(adam_step(h->compute, o));
-  h->main_images_stale = true;
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_stop, h->compute));
-  DRL_CUDA_CHECK(cudaEventRecord(h->ev_done, h->compute));
-  h->pending = true;
-  return DRL_OK;
+  return r2_backward(streams_of(h), h->pl, h->params, h->wi, h->grads, in, h->act, h->bwd, h->B, h->S, h->mode, launches);
 }
 
 // H2D of nb sequences into slot s on `stream` (fields that are null are skipped)
-int stage_into(drl_r2d2* h, R2Slot& s, cudaStream_t stream, int nb, int steps, const uint8_t* state,
+int stage_into(drl_r2d2* h, R2In& s, cudaStream_t stream, int nb, int steps, const uint8_t* state,
                const int32_t* previous_action, const int32_t* action, const float* h0, const float* c0, const float* reward,
                const uint8_t* done, const float* weight) {
   auto cp = [&](const void* dst, const void* src, size_t bytes) -> cudaError_t {
     return cudaMemcpyAsync(const_cast<void*>(dst), src, bytes, cudaMemcpyHostToDevice, stream);
   };
   const size_t n = (size_t)nb * steps;
-  DRL_CUDA_CHECK(cp(s.in.frames, state, n * h->frame));
-  DRL_CUDA_CHECK(cp(s.in.pa, previous_action, n * 4));
-  if (action) DRL_CUDA_CHECK(cp(s.in.action, action, n * 4));
-  DRL_CUDA_CHECK(cp(s.in.h0, h0, (size_t)nb * kR2L * 4));
-  DRL_CUDA_CHECK(cp(s.in.c0, c0, (size_t)nb * kR2L * 4));
-  if (reward) DRL_CUDA_CHECK(cp(s.in.reward, reward, n * 4));
-  if (done) DRL_CUDA_CHECK(cp(s.in.done, done, n));
-  if (reward) DRL_CUDA_CHECK(cp(s.in.weight, weight ? weight : h->h_ones, (size_t)nb * 4));
+  DRL_CUDA_CHECK(cp(s.frames, state, n * h->frame));
+  DRL_CUDA_CHECK(cp(s.pa, previous_action, n * 4));
+  if (action) DRL_CUDA_CHECK(cp(s.action, action, n * 4));
+  DRL_CUDA_CHECK(cp(s.h0, h0, (size_t)nb * kR2L * 4));
+  DRL_CUDA_CHECK(cp(s.c0, c0, (size_t)nb * kR2L * 4));
+  if (reward) DRL_CUDA_CHECK(cp(s.reward, reward, n * 4));
+  if (done) DRL_CUDA_CHECK(cp(s.done, done, n));
+  if (reward) DRL_CUDA_CHECK(cp(s.weight, weight ? weight : h->h_ones, (size_t)nb * 4));
   return DRL_OK;
 }
 
@@ -935,25 +740,9 @@ int drl_r2d2_create(const drl_r2d2_config* cfg, drl_r2d2** out) {
   h->frame = (size_t)Geo::IH * Geo::IW * h->C;
   h->pl.init(h->A, h->C);
   int rc = [&]() -> int {
-    DRL_TRY(set_device(h));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->compute, cudaStreamNonBlocking));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->copy, cudaStreamNonBlocking));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking));
-    for (int i = 0; i < 8; ++i) DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->fj[i], cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->tmain, cudaStreamNonBlocking));
-    DRL_CUDA_CHECK(cudaStreamCreateWithFlags(&h->tside, cudaStreamNonBlocking));
-    for (int i = 0; i < 8; ++i) DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->tfj[i], cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_tfork, cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_tjoin, cudaEventDisableTiming));
-    DRL_CUDA_CHECK(cudaEventCreate(&h->ev_start));
-    DRL_CUDA_CHECK(cudaEventCreate(&h->ev_stop));
-    DRL_CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming));
-    const size_t B = h->B, S = h->S, M = B * S, A = h->A, NP = h->pl.padded_total;
-    DRL_TRY(dev_alloc(h, &h->params, NP));
-    DRL_TRY(dev_alloc(h, &h->target, NP));
-    DRL_TRY(dev_alloc(h, &h->adam_m, NP));
-    DRL_TRY(dev_alloc(h, &h->adam_v, NP));
-    DRL_TRY(dev_alloc(h, &h->grads, NP + 4));
+    const size_t B = h->B, S = h->S, M = B * S, A = h->A;
+    // constant learning rate (agent/r2d2.py:91); minimize(): no clipping
+    DRL_TRY(create_shell(h, M, AdamSchedule{cfg->learning_rate, cfg->learning_rate, 1.0, 0.0f}));
     DRL_TRY(alloc_acts(h, h->act));
     DRL_TRY(alloc_acts(h, h->tact));
     R2Bwd& b = h->bwd;
@@ -973,50 +762,13 @@ int drl_r2d2_create(const drl_r2d2_config* cfg, drl_r2d2** out) {
     DRL_TRY(dev_alloc(h, &b.wg_part, wg));
     DRL_TRY(dev_alloc(h, &b.wg_part2, wg));
     DRL_TRY(dev_alloc(h, &b.dcol, M * 81 * 512));
-    {
-      size_t wb[WeightImages::kCount];
-      weight_image_sizes(wb);
-      for (int i : {1, 2, 5, 6}) DRL_TRY(dev_alloc(h, &h->wi.img[i], wb[i]));
-      for (int i : {1, 2}) DRL_TRY(dev_alloc(h, &h->twi.img[i], wb[i]));
-    }
     const size_t Nt = h->Nt;
     DRL_TRY(dev_alloc(h, &h->sav, B * Nt));
     DRL_TRY(dev_alloc(h, &h->target_value, B * Nt));
     DRL_TRY(dev_alloc(h, &h->td_dev, B));
-    h->loss = h->grads + NP;     // loss scalar in the tail of the gradient bucket (one all-reduce covers both)
     DRL_TRY(dev_alloc(h, &h->c_last, M * kR2L));
-    DRL_TRY(dev_alloc(h, &h->d_step, 1));
-    DRL_TRY(dev_alloc(h, &h->d_lr, 1));
-    DRL_TRY(dev_alloc(h, &h->d_alpha, 1));
-    DRL_TRY(dev_alloc(h, &h->d_b1p, 1));
-    DRL_TRY(dev_alloc(h, &h->d_b2p, 1));
-    {
-      const float b1 = 0.9f, b2 = 0.999f;
-      DRL_CUDA_CHECK(cudaMemcpy(h->d_b1p, &b1, 4, cudaMemcpyHostToDevice));
-      DRL_CUDA_CHECK(cudaMemcpy(h->d_b2p, &b2, 4, cudaMemcpyHostToDevice));
-    }
-    const size_t ns = h->cfg.num_slots;
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_out, ns * 8 * sizeof(float), cudaHostAllocMapped));
-    DRL_CUDA_CHECK(cudaHostGetDevicePointer((void**)&h->d_out, h->h_out, 0));
-    memset(h->h_out, 0, ns * 8 * sizeof(float));
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_td, ns * B * sizeof(float), cudaHostAllocMapped));
-    DRL_CUDA_CHECK(cudaHostGetDevicePointer((void**)&h->d_td, h->h_td, 0));
-    memset(h->h_td, 0, ns * B * sizeof(float));
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_flat, NP * sizeof(float), cudaHostAllocDefault));
-    DRL_CUDA_CHECK(cudaHostAlloc((void**)&h->h_ones, M * sizeof(float), cudaHostAllocDefault));
-    for (size_t i = 0; i < M; ++i) h->h_ones[i] = 1.0f;
-    AdamState& o = h->opt;
-    o.params = h->params; o.m = h->adam_m; o.v = h->adam_v; o.grads = h->grads; o.n = (int64_t)NP;
-    o.nblk = 148 * 4;
-    DRL_TRY(dev_alloc(h, &o.norm_partials, o.nblk));
-    o.step = h->d_step; o.lr_cur = h->d_lr; o.alpha = h->d_alpha; o.b1p = h->d_b1p; o.b2p = h->d_b2p;
-    o.out = h->d_out; o.loss = h->loss;
-    o.start_lr = cfg->learning_rate; o.end_lr = cfg->learning_rate; o.learning_frame = 1.0;   // constant (agent/r2d2.py:91)
-    o.clip_norm = 0.0f;                                                                        // minimize(): no clipping
-    o.grad_scale = 1.0f;
-    h->slots.resize(ns + 1);
-    h->graph_step.assign(ns, nullptr);
-    for (R2Slot& s : h->slots) {
+    h->slots.resize(h->sync.size());
+    for (R2In& s : h->slots) {
       size_t off = 0;
       const size_t o_fr = off; off = align_up(off + M * h->frame, 256);
       const size_t o_pa = off; off = align_up(off + M * 4, 256);
@@ -1026,196 +778,92 @@ int drl_r2d2_create(const drl_r2d2_config* cfg, drl_r2d2** out) {
       const size_t o_rw = off; off = align_up(off + M * 4, 256);
       const size_t o_dn = off; off = align_up(off + M, 256);
       const size_t o_wt = off; off = align_up(off + M * 4, 256);
-      DRL_TRY(dev_alloc(h, &s.base, off));
-      s.in.frames = s.base + o_fr;
-      s.in.pa = reinterpret_cast<int32_t*>(s.base + o_pa);
-      s.in.action = reinterpret_cast<int32_t*>(s.base + o_ac);
-      s.in.h0 = reinterpret_cast<float*>(s.base + o_h);
-      s.in.c0 = reinterpret_cast<float*>(s.base + o_c);
-      s.in.reward = reinterpret_cast<float*>(s.base + o_rw);
-      s.in.done = s.base + o_dn;
-      s.in.weight = reinterpret_cast<float*>(s.base + o_wt);
-      DRL_CUDA_CHECK(cudaEventCreateWithFlags(&s.staged, cudaEventDisableTiming));
-      DRL_CUDA_CHECK(cudaEventCreateWithFlags(&s.consumed, cudaEventDisableTiming));
+      uint8_t* base = nullptr;
+      DRL_TRY(dev_alloc(h, &base, off));
+      s.frames = base + o_fr;
+      s.pa = reinterpret_cast<int32_t*>(base + o_pa);
+      s.action = reinterpret_cast<int32_t*>(base + o_ac);
+      s.h0 = reinterpret_cast<float*>(base + o_h);
+      s.c0 = reinterpret_cast<float*>(base + o_c);
+      s.reward = reinterpret_cast<float*>(base + o_rw);
+      s.done = base + o_dn;
+      s.weight = reinterpret_cast<float*>(base + o_wt);
     }
     DRL_CUDA_CHECK(cudaDeviceSynchronize());
     return DRL_OK;
   }();
-  if (rc != DRL_OK) {
-    std::string keep = get_error();
-    drl_r2d2_destroy(h);
-    set_error("%s", keep.c_str());
-    return rc;
-  }
-  *out = h;
-  return DRL_OK;
+  return finish_create(h, rc, out);
 }
 
-int drl_r2d2_destroy(drl_r2d2* h) {
-  if (!h) return DRL_OK;
-  cudaSetDevice(h->cfg.device);
-  cudaDeviceSynchronize();
-  for (auto g : h->graph_step) if (g) cudaGraphExecDestroy(g);
-  for (R2Slot& s : h->slots) {
-    if (s.staged) cudaEventDestroy(s.staged);
-    if (s.consumed) cudaEventDestroy(s.consumed);
-  }
-  for (void* p : h->allocs) cudaFree(p);
-  if (h->h_out) cudaFreeHost(h->h_out);
-  if (h->h_td) cudaFreeHost(h->h_td);
-  if (h->h_flat) cudaFreeHost(h->h_flat);
-  if (h->h_ones) cudaFreeHost(h->h_ones);
-  if (h->ev_start) cudaEventDestroy(h->ev_start);
-  if (h->ev_stop) cudaEventDestroy(h->ev_stop);
-  if (h->ev_done) cudaEventDestroy(h->ev_done);
-  for (int i = 0; i < 8; ++i) if (h->fj[i]) cudaEventDestroy(h->fj[i]);
-  for (int i = 0; i < 8; ++i) if (h->tfj[i]) cudaEventDestroy(h->tfj[i]);
-  if (h->ev_tfork) cudaEventDestroy(h->ev_tfork);
-  if (h->ev_tjoin) cudaEventDestroy(h->ev_tjoin);
-  if (h->tmain) cudaStreamDestroy(h->tmain);
-  if (h->tside) cudaStreamDestroy(h->tside);
-  if (h->side) cudaStreamDestroy(h->side);
-  if (h->compute) cudaStreamDestroy(h->compute);
-  if (h->copy) cudaStreamDestroy(h->copy);
-  cudaGetLastError();
-  delete h;
-  return DRL_OK;
-}
+int drl_r2d2_destroy(drl_r2d2* h) { return destroy_shell(h); }
 
 int drl_r2d2_param_count(const drl_r2d2* h, int64_t* n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
+  DRL_ENTER(h);
   if (!n) { set_error("null argument"); return DRL_ERR_INVALID; }
   *n = h->pl.packed_total;
   return DRL_OK;
 }
 int drl_r2d2_set_params(drl_r2d2* h, int32_t which, const float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (which != 0 && which != 1) { set_error("which must be 0 (main) or 1 (target)"); return DRL_ERR_INVALID; }
-  if (!host_flat || n != h->pl.packed_total) { set_error("set_params: expected %lld floats, got %lld", (long long)h->pl.packed_total, (long long)n); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_TRY(upload_flat(h, which == 0 ? h->params : h->target, host_flat));
-  if (which == 0) h->main_images_stale = true; else h->target_images_stale = true;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return set_params(h, which, host_flat, n);
 }
 int drl_r2d2_get_params(drl_r2d2* h, int32_t which, float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (which != 0 && which != 1) { set_error("which must be 0 (main) or 1 (target)"); return DRL_ERR_INVALID; }
-  if (!host_flat || n != h->pl.packed_total) { set_error("get_params: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return download_flat(h, which == 0 ? h->params : h->target, host_flat);
+  DRL_ENTER(h);
+  return get_params(h, which, host_flat, n);
 }
 int drl_r2d2_set_opt_state(drl_r2d2* h, const float* host_m, const float* host_v, int64_t n, int64_t step,
                            float beta1_power, float beta2_power) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (!host_m || !host_v || n != h->pl.packed_total) { set_error("set_opt_state: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_TRY(upload_flat(h, h->adam_m, host_m));
-  DRL_TRY(upload_flat(h, h->adam_v, host_v));
-  long long st = step;
-  DRL_CUDA_CHECK(cudaMemcpy(h->d_step, &st, sizeof(st), cudaMemcpyHostToDevice));
-  DRL_CUDA_CHECK(cudaMemcpy(h->d_b1p, &beta1_power, 4, cudaMemcpyHostToDevice));
-  DRL_CUDA_CHECK(cudaMemcpy(h->d_b2p, &beta2_power, 4, cudaMemcpyHostToDevice));
-  return DRL_OK;
+  DRL_ENTER(h);
+  return set_opt_state(h, host_m, host_v, n, step, beta1_power, beta2_power);
 }
 int drl_r2d2_get_opt_state(drl_r2d2* h, float* host_m, float* host_v, int64_t n, int64_t* step, float* beta1_power,
                            float* beta2_power) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (n != h->pl.packed_total) { set_error("get_opt_state: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  if (host_m) DRL_TRY(download_flat(h, h->adam_m, host_m));
-  if (host_v) DRL_TRY(download_flat(h, h->adam_v, host_v));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  if (step) {
-    long long st = 0;
-    DRL_CUDA_CHECK(cudaMemcpy(&st, h->d_step, sizeof(st), cudaMemcpyDeviceToHost));
-    *step = st;
-  }
-  if (beta1_power) DRL_CUDA_CHECK(cudaMemcpy(beta1_power, h->d_b1p, 4, cudaMemcpyDeviceToHost));
-  if (beta2_power) DRL_CUDA_CHECK(cudaMemcpy(beta2_power, h->d_b2p, 4, cudaMemcpyDeviceToHost));
-  return DRL_OK;
+  DRL_ENTER(h);
+  return get_opt_state(h, host_m, host_v, n, step, beta1_power, beta2_power);
 }
 int drl_r2d2_get_grads(drl_r2d2* h, float* host_flat, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (!host_flat || n != h->pl.packed_total) { set_error("get_grads: expected %lld floats", (long long)h->pl.packed_total); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return download_flat(h, h->grads, host_flat);
+  DRL_ENTER(h);
+  return get_grads(h, host_flat, n);
 }
 int drl_r2d2_main_to_target(drl_r2d2* h) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  DRL_TRY(set_device(h));
-  DRL_CUDA_CHECK(cudaMemcpyAsync(h->target, h->params, h->pl.padded_total * sizeof(float), cudaMemcpyDeviceToDevice, h->compute));
-  pdl_break(h->compute);
-  h->target_images_stale = true;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return copy_main_to_target(h);
 }
 
 int drl_r2d2_stage(drl_r2d2* h, int32_t slot, const uint8_t* state, const int32_t* previous_action, const int32_t* action,
                    const float* h0, const float* c0, const float* reward, const uint8_t* done, const float* weight) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
+  DRL_ENTER(h);
   if (!state || !previous_action || !action || !h0 || !c0 || !reward || !done) { set_error("stage: null input pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  R2Slot& s = h->slots[slot];
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->copy, s.consumed, 0));
-  DRL_TRY(stage_into(h, s, h->copy, h->B, h->S, state, previous_action, action, h0, c0, reward, done, weight));
-  DRL_CUDA_CHECK(cudaEventRecord(s.staged, h->copy));
-  s.has_data = true;
-  return DRL_OK;
+  return stage_slot(h, slot, [&](cudaStream_t s) {
+    return stage_into(h, h->slots[slot], s, h->B, h->S, state, previous_action, action, h0, c0, reward, done, weight);
+  });
 }
 
 int drl_r2d2_step_async(drl_r2d2* h, int32_t slot) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return run_step(h, slot);
+  DRL_ENTER(h);
+  return run_step(h, slot, forward_backward);
 }
 int drl_r2d2_forward_backward(drl_r2d2* h, int32_t slot) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  return run_forward_backward(h, slot);
+  DRL_ENTER(h);
+  return run_forward_backward(h, slot, forward_backward);
 }
 int drl_r2d2_grad_bucket(drl_r2d2* h, void** dev_ptr, int64_t* count) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (dev_ptr) *dev_ptr = h->grads;
-  if (count) *count = h->pl.padded_total + 4;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return grad_bucket(h, dev_ptr, count);
 }
 int drl_r2d2_apply(drl_r2d2* h, float grad_scale) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (!(grad_scale > 0.f)) { set_error("apply: grad_scale must be > 0"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
+  DRL_ENTER(h);
   return run_apply(h, grad_scale);
 }
 int drl_r2d2_wait(drl_r2d2* h, drl_r2d2_out* out, float* td_error) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (!h->pending) { set_error("wait: no step in flight"); return DRL_ERR_STATE; }
-  DRL_TRY(set_device(h));
-  h->pending = false;
-  DRL_CUDA_CHECK(cudaEventSynchronize(h->ev_done));
-  const float* r = h->h_out + 8 * h->last_slot;
+  DRL_ENTER(h);
+  const float* r = nullptr;
+  DRL_TRY(wait_step(h, td_error, &r));
   if (out) {
     out->loss = r[0];
     out->grad_norm = r[2];
-    uint32_t lo, hi;
-    memcpy(&lo, &r[6], 4);
-    memcpy(&hi, &r[7], 4);
-    out->step = (int64_t)(((uint64_t)hi << 32) | lo);
+    out->step = result_row_step(r);
   }
-  if (td_error) memcpy(td_error, h->h_td + (size_t)h->last_slot * h->B, (size_t)h->B * sizeof(float));
   return DRL_OK;
 }
 int drl_r2d2_step(drl_r2d2* h, int32_t slot, drl_r2d2_out* out, float* td_error) {
@@ -1225,35 +873,31 @@ int drl_r2d2_step(drl_r2d2* h, int32_t slot, drl_r2d2_out* out, float* td_error)
 
 int drl_r2d2_td_error(drl_r2d2* h, int32_t n, const uint8_t* state, const int32_t* previous_action, const int32_t* action,
                       const float* h0, const float* c0, const float* reward, const uint8_t* done, float* td_error) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
+  DRL_ENTER(h);
   if (n < 1 || n > h->B) { set_error("td_error: n must be in [1, %d]", h->B); return DRL_ERR_INVALID; }
   if (!state || !previous_action || !action || !h0 || !c0 || !reward || !done || !td_error) { set_error("td_error: null pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  R2Slot& s = h->slots[h->cfg.num_slots];
+  R2In& s = h->slots[h->cfg.num_slots];
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
   DRL_TRY(stage_into(h, s, h->compute, n, h->S, state, previous_action, action, h0, c0, reward, done, nullptr));
-  DRL_TRY(enqueue_forward_td(h, s.in, n, false, nullptr, nullptr));
+  DRL_TRY(enqueue_forward_td(h, s, n, false, nullptr, nullptr));
   DRL_CUDA_CHECK(cudaMemcpyAsync(td_error, h->td_dev, (size_t)n * 4, cudaMemcpyDeviceToHost, h->compute));
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  h->last_b = n;
+  h->last_rows = n;
   return DRL_OK;
 }
 
 int drl_r2d2_act(drl_r2d2* h, int32_t n, const uint8_t* state, const int32_t* previous_action, const float* h_in,
                  const float* c_in, float* q_value, float* h_out, float* c_out) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
+  DRL_ENTER(h);
   const int M = h->B * h->S;
   if (n < 1 || n > M) { set_error("act: n must be in [1, %d]", M); return DRL_ERR_INVALID; }
   if (!state || !previous_action || !h_in || !c_in) { set_error("act: null pointer"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  R2Slot& s = h->slots[h->cfg.num_slots];
+  R2In& s = h->slots[h->cfg.num_slots];
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
   DRL_TRY(stage_into(h, s, h->compute, n, 1, state, previous_action, nullptr, h_in, c_in, nullptr, nullptr, nullptr));
   pdl_break(h->compute);
   pdl_break(h->side);
-  R2In in = s.in;
+  R2In in = s;
   in.done = nullptr;                                     // a single step: nothing is carried
   DRL_TRY(r2_forward(streams_of(h), h->pl, h->params, h->wi, in, h->act, h->c_last, n, 1, h->mode, h->main_images_stale,
                      h->main_images_stale, false, nullptr));
@@ -1262,17 +906,15 @@ int drl_r2d2_act(drl_r2d2* h, int32_t n, const uint8_t* state, const int32_t* pr
   if (h_out) DRL_CUDA_CHECK(cudaMemcpyAsync(h_out, h->act.hout, (size_t)n * kR2L * 4, cudaMemcpyDeviceToHost, h->compute));
   if (c_out) DRL_CUDA_CHECK(cudaMemcpyAsync(c_out, h->c_last, (size_t)n * kR2L * 4, cudaMemcpyDeviceToHost, h->compute));
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  h->last_b = 0;
+  h->last_rows = 0;
   return DRL_OK;
 }
 
 int drl_r2d2_taps(drl_r2d2* h, float* main_q, float* target_q, float* target_value, float* state_action_value) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  DRL_TRY(set_device(h));
-  if (h->last_b < 1) { set_error("taps: no step or td_error call has run"); return DRL_ERR_STATE; }
+  DRL_ENTER(h);
+  if (h->last_rows < 1) { set_error("taps: no step or td_error call has run"); return DRL_ERR_STATE; }
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  const int nb = h->last_b, S = h->S, A = h->A;
+  const int nb = h->last_rows, S = h->S, A = h->A;
   // time-major device rows -> batch-major host arrays [nb, S, A]
   for (int which = 0; which < 2; ++which) {
     float* dst = which == 0 ? main_q : target_q;
@@ -1290,73 +932,36 @@ int drl_r2d2_taps(drl_r2d2* h, float* main_q, float* target_q, float* target_val
 }
 
 int drl_r2d2_read_buffer(drl_r2d2* h, const char* name, float* host_dst, int64_t n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
+  DRL_ENTER(h);
   if (!name || !host_dst) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  if (h->last_b < 1) { set_error("read_buffer: no step or td_error call has run"); return DRL_ERR_STATE; }
-  const size_t M = (size_t)h->last_b * h->S, A = h->A;
-  struct Ent { const char* nm; const float* p; size_t cnt; };
-  const Ent tab[] = {
+  if (h->last_rows < 1) { set_error("read_buffer: no step or td_error call has run"); return DRL_ERR_STATE; }
+  const size_t M = (size_t)h->last_rows * h->S, A = h->A;
+  const NamedBuffer tab[] = {
       {"a1", h->act.a1, M * 400 * 32}, {"a2", h->act.a2, M * 81 * 64}, {"a3", h->act.a3, M * Geo::FLAT},
       {"emb", h->act.table, A * Geo::EMB}, {"e1", h->act.e1, A * Geo::EMB}, {"q1", h->act.q1, M * kR2H},
       {"hout", h->act.hout, M * kR2L}, {"hin", h->act.hin, M * kR2L}, {"cin", h->act.cin, M * kR2L},
       {"gates", h->act.gates, M * kR2G}, {"dz", h->bwd.dz, M * kR2G}, {"dhout", h->bwd.dhout, M * kR2L},
       {"da3", h->bwd.da3, M * Geo::FLAT}};
-  for (const Ent& e : tab) {
-    if (strcmp(e.nm, name) == 0) {
-      if ((size_t)n != e.cnt) { set_error("read_buffer(%s): expected %zu floats, got %lld", name, e.cnt, (long long)n); return DRL_ERR_INVALID; }
-      DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-      DRL_CUDA_CHECK(cudaMemcpy(host_dst, e.p, e.cnt * sizeof(float), cudaMemcpyDeviceToHost));
-      return DRL_OK;
-    }
-  }
-  set_error("read_buffer: unknown buffer '%s'", name);
-  return DRL_ERR_INVALID;
+  return read_named_buffer(h->compute, tab, sizeof(tab) / sizeof(tab[0]), name, host_dst, n);
 }
 
 int drl_r2d2_profile_step(drl_r2d2* h, int32_t slot, char* names, int64_t names_len, float* ms, int32_t max_kernels,
                           int32_t* count) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (slot < 0 || slot >= h->cfg.num_slots) { set_error("slot %d out of range", slot); return DRL_ERR_INVALID; }
-  if (!names || !ms || !count) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  R2Slot& sl = h->slots[slot];
-  if (!sl.has_data) { set_error("slot %d has not been staged", slot); return DRL_ERR_STATE; }
-  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, sl.staged, 0));
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  prof_begin();
-  const bool par_saved = h->par;
-  h->par = false;
-  h->main_images_stale = true;
-  int rc = enqueue_step(h, slot, nullptr);
-  h->par = par_saved;
-  h->main_images_stale = true;
-  h->last_b = h->B;
-  DRL_TRY(prof_end(h->compute, rc, names, names_len, ms, max_kernels, count));
-  h->pending = false;
-  return DRL_OK;
+  DRL_ENTER(h);
+  return profile_step(h, slot, forward_backward, names, names_len, ms, max_kernels, count);
 }
 int drl_r2d2_last_step_ms(drl_r2d2* h, float* ms) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
-  if (!ms) { set_error("null argument"); return DRL_ERR_INVALID; }
-  DRL_TRY(set_device(h));
-  DRL_CUDA_CHECK(cudaEventSynchronize(h->ev_stop));
-  DRL_CUDA_CHECK(cudaEventElapsedTime(ms, h->ev_start, h->ev_stop));
-  return DRL_OK;
+  DRL_ENTER(h);
+  return last_step_ms(h, ms);
 }
 int drl_r2d2_stream(drl_r2d2* h, void** stream) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
+  DRL_ENTER(h);
   if (!stream) { set_error("null argument"); return DRL_ERR_INVALID; }
   *stream = h->compute;
   return DRL_OK;
 }
 int drl_r2d2_launches_per_step(const drl_r2d2* h, int32_t* n) {
-  DRL_TRY(check_handle(h));
-  std::lock_guard<std::recursive_mutex> _lk(const_cast<drl_r2d2*>(h)->mu);
+  DRL_ENTER(h);
   if (!n) { set_error("null argument"); return DRL_ERR_INVALID; }
   *n = h->launches;
   return DRL_OK;

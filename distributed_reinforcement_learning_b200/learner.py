@@ -13,18 +13,14 @@ import ctypes as C
 import numpy as np
 
 from . import _native as N
+from ._native import _as_u8
 
 H, W, CH, LSTM = 84, 84, 4, 256
 
 
-def _as_u8(done):
-    d = np.asarray(done)
-    if d.dtype == np.bool_:
-        return np.ascontiguousarray(d).view(np.uint8)      # bool is one byte, 0/1: no copy
-    return d.astype(np.uint8, copy=False)
+class NativeLearner(N.NativeHandle):
+    _prefix = "learner"
 
-
-class NativeLearner:
     def __init__(self, batch, trajectory=20, num_action=18, lstm_hidden_size=256, input_shape=(84, 84, 4),
                  discount_factor=0.99, start_learning_rate=0.0006, end_learning_rate=0.0,
                  learning_frame=1000000000, baseline_loss_coef=1.0, entropy_coef=0.05,
@@ -40,40 +36,13 @@ class NativeLearner:
                               end_learning_rate, float(learning_frame), baseline_loss_coef, entropy_coef,
                               gradient_clip_norm, N.REWARD_CLIPPING[reward_clipping], self.device, int(num_slots),
                               int(bool(use_cuda_graph)), int(math_mode))
-        self._h = C.c_void_p()
-        N.check(N.lib.drl_learner_create(C.byref(cfg), C.byref(self._h)))
-        n = C.c_int64()
-        N.check(N.lib.drl_learner_param_count(self._h, C.byref(n)))
-        self.param_count = int(n.value)
-        self.num_slots = int(num_slots)
-        self._keep = [None] * self.num_slots     # host arrays referenced by in-flight H2D copies
+        self._open(cfg, num_slots)
         self._bucket = None
         self._ext_stream = None
         self._peer = False
         self._no_collective = False          # diagnostic only (bench.py --collective none)
 
-    # ---- lifetime ----------------------------------------------------------------
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            N.lib.drl_learner_destroy(self._h)
-            self._h = C.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    # ---- parameters / optimizer state ---------------------------------------------
-    def set_params(self, flat):
-        a = N.as_c(flat, np.float32, (self.param_count,), "params")
-        N.check(N.lib.drl_learner_set_params(self._h, N.ptr(a), a.size))
-
-    def get_params(self):
-        a = np.empty(self.param_count, np.float32)
-        N.check(N.lib.drl_learner_get_params(self._h, N.ptr(a), a.size))
-        return a
-
+    # ---- optimizer state ---------------------------------------------------------------
     def set_opt_state(self, ms_flat, step):
         a = N.as_c(ms_flat, np.float32, (self.param_count,), "ms")
         N.check(N.lib.drl_learner_set_opt_state(self._h, N.ptr(a), a.size, int(step)))
@@ -83,11 +52,6 @@ class NativeLearner:
         st = C.c_int64()
         N.check(N.lib.drl_learner_get_opt_state(self._h, N.ptr(a), a.size, C.byref(st)))
         return a, int(st.value)
-
-    def get_grads(self):
-        a = np.empty(self.param_count, np.float32)
-        N.check(N.lib.drl_learner_get_grads(self._h, N.ptr(a), a.size))
-        return a
 
     # ---- data path -----------------------------------------------------------------
     def stage(self, slot, state, reward, action, done, behavior_policy, previous_action, initial_h, initial_c):
@@ -156,11 +120,6 @@ class NativeLearner:
         N.check(N.lib.drl_learner_taps(self._h, *[N.ptr(a) for a in out]))
         return dict(vs=out[0], clipped_rho=out[1], vs_plus_1=out[2], pg_advantage=out[3])
 
-    def read_buffer(self, name, count):
-        a = np.empty(int(count), np.float32)
-        N.check(N.lib.drl_learner_read_buffer(self._h, name.encode(), N.ptr(a), a.size))
-        return a
-
     def act(self, state, previous_action, h, c):
         """n single-step forwards (agent/impala.py:118-130 without the sampling)."""
         st = N.as_c(state, np.uint8)
@@ -175,31 +134,6 @@ class NativeLearner:
         N.check(N.lib.drl_learner_act(self._h, n, N.ptr(st), N.ptr(pa), N.ptr(hh), N.ptr(cc), N.ptr(pol),
                                       N.ptr(ho), N.ptr(co)))
         return pol, ho, co
-
-    def profile_step(self, slot=0, max_kernels=128):
-        """One real step with a CUDA event before every launch -> [(kernel name, device ms)]."""
-        names = C.create_string_buffer(8192)
-        ms = np.zeros(max_kernels, np.float32)
-        cnt = C.c_int32()
-        N.check(N.lib.drl_learner_profile_step(self._h, slot, names, len(names), N.ptr(ms), max_kernels,
-                                               C.byref(cnt)))
-        nm = names.value.decode().split("\n") if cnt.value else []
-        return list(zip(nm, [float(x) for x in ms[:cnt.value]]))
-
-    def last_step_ms(self):
-        ms = C.c_float()
-        N.check(N.lib.drl_learner_last_step_ms(self._h, C.byref(ms)))
-        return float(ms.value)
-
-    def launches_per_step(self):
-        n = C.c_int32()
-        N.check(N.lib.drl_learner_launches_per_step(self._h, C.byref(n)))
-        return int(n.value)
-
-    def stream_ptr(self):
-        s = C.c_void_p()
-        N.check(N.lib.drl_learner_stream(self._h, C.byref(s)))
-        return int(s.value or 0)
 
     # ---- data parallel ---------------------------------------------------------------
     @staticmethod
