@@ -53,12 +53,18 @@ def adam_expected(p0, g, m0, v0, gn, clip, lr, b1p, b2p):
     return p0 - m * alpha / (np.sqrt(v) + ax.ADAM_EPS), m, v
 
 
-def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", sync_target_at=None, **kw):
+def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", sync_target_at=None, gradient_clip_norm=None,
+                 learning_frame=None, end_learning_rate=None, **kw):
+    """``gradient_clip_norm`` / ``learning_frame`` / ``end_learning_rate``: optional, for both the oracle and the native
+    learner (the configuration defaults otherwise); with a clip norm given, ``clip_engaged`` entries are 0 where the
+    step's norm exceeded it and inf where it did not."""
     params = ax.init_params(0, torch.float32, num_action=A)
     target = ax.init_params(1, torch.float32, num_action=A)
+    schedule = {k: v for k, v in (("gradient_clip_norm", gradient_clip_norm), ("learning_frame", learning_frame),
+                                  ("end_learning_rate", end_learning_rate)) if v is not None}
     cfg = dict(num_action=A, reward_clipping=reward_clipping)
-    L = ax.Learner(params, target, torch.float64, **cfg)
-    eng = native_apex(B, A, params, target, reward_clipping=reward_clipping, **kw)
+    L = ax.Learner(params, target, torch.float64, **cfg, **schedule)
+    eng = native_apex(B, A, params, target, reward_clipping=reward_clipping, **schedule, **kw)
     errs = {}
     flips = elems = 0
     max_abs = 0.0
@@ -94,6 +100,8 @@ def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", sync_tar
             errs["td_error" + tag] = rel_err(td, res[1])
             errs["lr" + tag] = abs(out["learning_rate"] - lr)
             errs["grad_norm" + tag] = rel_err(out["grad_norm"], gn)
+            if gradient_clip_norm is not None:
+                errs["clip_engaged" + tag] = 0.0 if gn > gradient_clip_norm else float("inf")
             if out["step"] != s + 1:
                 errs["step" + tag] = float("inf")
             for k in ("main_q", "next_main_q", "target_q", "target_value", "state_action_value"):
@@ -119,8 +127,8 @@ def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", sync_tar
             gn_gpu = float(np.sqrt(np.sum(g_gpu_flat.astype(np.float64) ** 2)))
             exp_p, exp_m, exp_v = adam_expected(p0.astype(np.float64), g_gpu_flat.astype(np.float64),
                                                 st0["m"].astype(np.float64), st0["v"].astype(np.float64), gn_gpu,
-                                                40.0, float(out["learning_rate"]), st0["beta1_power"],
-                                                st0["beta2_power"])
+                                                L.cfg["gradient_clip_norm"], float(out["learning_rate"]),
+                                                st0["beta1_power"], st0["beta2_power"])
             floor = 4.0 * np.finfo(np.float32).eps * np.max(np.abs(p0)) / TOL
             errs["update/adam" + tag] = float(np.max(np.abs(p1 - exp_p)) / (np.max(np.abs(exp_p - p0)) + floor))
             errs["adam/m" + tag] = rel_err(st1["m"], exp_m)

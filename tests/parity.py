@@ -49,10 +49,17 @@ def to_batch_major(x_m, B, T):
     return np.swapaxes(x.reshape((T, B) + x.shape[1:]), 0, 1).reshape((B * T,) + x.shape[1:])
 
 
-def make_case(B, T=20, A=18, seed=1234, param_seed=0, reward_clipping="abs_one"):
+SCHEDULE_KEYS = ("gradient_clip_norm", "learning_frame", "end_learning_rate")
+
+
+def make_case(B, T=20, A=18, seed=1234, param_seed=0, reward_clipping="abs_one", **schedule):
+    """``schedule``: optional gradient_clip_norm / learning_frame / end_learning_rate for both the oracle and the
+    native learner (the configuration defaults otherwise)."""
+    assert set(schedule) <= set(SCHEDULE_KEYS), schedule
     batch = synthetic.make_batch(B, T=T, A=A, seed=seed)
     params = it.init_params(param_seed, torch.float32, num_action=A)
-    cfg = dict(trajectory=T, num_action=A, reward_clipping=reward_clipping)
+    cfg = dict(trajectory=T, num_action=A, reward_clipping=reward_clipping,
+               **{k: v for k, v in schedule.items() if v is not None})
     return batch, params, cfg
 
 
@@ -60,7 +67,8 @@ def native_learner(batch, params, cfg, **kw):
     from distributed_reinforcement_learning_b200.learner import NativeLearner
     B = batch["state"].shape[0]
     eng = NativeLearner(batch=B, trajectory=cfg["trajectory"], num_action=cfg["num_action"],
-                        reward_clipping=cfg.get("reward_clipping", "abs_one"), **kw)
+                        reward_clipping=cfg.get("reward_clipping", "abs_one"),
+                        **{k: cfg[k] for k in SCHEDULE_KEYS if k in cfg}, **kw)
     eng.set_params(it.flatten_params(params))
     return eng
 
@@ -83,11 +91,15 @@ def gpu_activation_pattern(eng, B, T, A):
     return masks
 
 
-def compare_step(B, T=20, A=18, seed=1234, steps=1, reward_clipping="abs_one", layers=True, **kw):
+def compare_step(B, T=20, A=18, seed=1234, steps=1, reward_clipping="abs_one", layers=True, gradient_clip_norm=None,
+                 learning_frame=None, end_learning_rate=None, **kw):
     """Returns {name: rel_err} for activations, taps, losses, every parameter gradient, and the applied
     update / RMSProp slots after each of `steps` updates (GPU step first, then the float64 oracle step
-    evaluated at the GPU's ReLU activation pattern)."""
-    batch, params, cfg = make_case(B, T, A, seed, reward_clipping=reward_clipping)
+    evaluated at the GPU's ReLU activation pattern).  With ``gradient_clip_norm`` given, ``clip_engaged`` entries
+    are 0 where the step's norm exceeded it and inf where it did not."""
+    batch, params, cfg = make_case(B, T, A, seed, reward_clipping=reward_clipping,
+                                   gradient_clip_norm=gradient_clip_norm, learning_frame=learning_frame,
+                                   end_learning_rate=end_learning_rate)
     L = it.Learner(params, torch.float64, "dedup", **cfg)
     eng = native_learner(batch, params, cfg, **kw)
     args = [batch[k] for k in synthetic.TRAIN_FIELDS]
@@ -109,6 +121,8 @@ def compare_step(B, T=20, A=18, seed=1234, steps=1, reward_clipping="abs_one", l
                 errs["loss/" + k + tag] = rel_err(out[k], float(o[k].detach()))
             errs["lr" + tag] = abs(out["learning_rate"] - res[3])
             errs["grad_norm" + tag] = rel_err(out["grad_norm"], gn)
+            if gradient_clip_norm is not None:
+                errs["clip_engaged" + tag] = 0.0 if gn > gradient_clip_norm else float("inf")
             if out["step"] != s + 1:
                 errs["step" + tag] = float("inf")
             taps = eng.taps()

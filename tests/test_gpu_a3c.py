@@ -17,11 +17,15 @@ def _masks(eng, B, A):
     return {k.replace("value", "actor").replace("mean", "critic"): v for k, v in m.items()}
 
 
-def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", **kw):
+def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", gradient_clip_norm=None, learning_frame=None,
+                 end_learning_rate=None, **kw):
+    """The schedule arguments are optional and reach both learners, as in apex_parity.compare_step."""
     from distributed_reinforcement_learning_b200.a3c_learner import NativeA3CLearner
     params = at.init_params(0, torch.float32, num_action=A)
-    L = at.Learner(params, torch.float64, num_action=A, reward_clipping=reward_clipping)
-    eng = NativeA3CLearner(batch=B, num_action=A, reward_clipping=reward_clipping, **kw)
+    schedule = {k: v for k, v in (("gradient_clip_norm", gradient_clip_norm), ("learning_frame", learning_frame),
+                                  ("end_learning_rate", end_learning_rate)) if v is not None}
+    L = at.Learner(params, torch.float64, num_action=A, reward_clipping=reward_clipping, **schedule)
+    eng = NativeA3CLearner(batch=B, num_action=A, reward_clipping=reward_clipping, **schedule, **kw)
     eng.set_params(at.flatten_params(params))
     errs = {}
     flips = elems = 0
@@ -42,6 +46,8 @@ def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", **kw):
                 errs["loss/" + k + tag] = rel_err(out[k], res[i])
             errs["lr" + tag] = abs(out["learning_rate"] - res[3])
             errs["grad_norm" + tag] = rel_err(out["grad_norm"], gn)
+            if gradient_clip_norm is not None:
+                errs["clip_engaged" + tag] = 0.0 if gn > gradient_clip_norm else float("inf")
             if out["step"] != s + 1:
                 errs["step" + tag] = float("inf")
             for k in ("policy", "value", "next_value", "advantage"):
@@ -53,7 +59,8 @@ def compare_step(B, A=4, seed=4321, steps=1, reward_clipping="abs_one", **kw):
             st1, p1 = eng.get_opt_state(), eng.get_params()
             g64 = g_gpu.astype(np.float64)
             exp_p, exp_m, exp_v = ap.adam_expected(p0.astype(np.float64), g64, st0["m"].astype(np.float64),
-                                                   st0["v"].astype(np.float64), float(np.sqrt(np.sum(g64 ** 2))), 40.0,
+                                                   st0["v"].astype(np.float64), float(np.sqrt(np.sum(g64 ** 2))),
+                                                   L.cfg["gradient_clip_norm"],
                                                    float(out["learning_rate"]), st0["beta1_power"], st0["beta2_power"])
             floor = 4.0 * np.finfo(np.float32).eps * np.max(np.abs(p0)) / TOL
             errs["update/adam" + tag] = float(np.max(np.abs(p1 - exp_p)) / (np.max(np.abs(exp_p - p0)) + floor))
