@@ -213,6 +213,16 @@ def _load():
         "drl_per_total": (C.c_int, [vp, C.POINTER(C.c_double)]),
         "drl_per_size": (C.c_int, [vp, C.POINTER(i64)]),
         "drl_per_beta": (C.c_int, [vp, C.POINTER(C.c_double)]),
+        "drl_apex_replay_create": (C.c_int, [vp, i64, C.c_uint64, C.POINTER(vp)]),
+        "drl_apex_replay_destroy": (C.c_int, [vp]),
+        "drl_apex_replay_add": (C.c_int, [vp, i32] + [vp] * 6),
+        "drl_apex_replay_step_async": (C.c_int, [vp, i32]),
+        "drl_apex_replay_step": (C.c_int, [vp, i32, C.POINTER(ApexOut), vp]),
+        "drl_apex_replay_last_sample": (C.c_int, [vp] * 5),
+        "drl_apex_replay_last_update": (C.c_int, [vp, vp, vp, i32, C.POINTER(i32)]),
+        "drl_apex_replay_info": (C.c_int, [vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(C.c_double),
+                                           C.POINTER(C.c_double), C.POINTER(i64)]),
+        "drl_apex_replay_read_tree": (C.c_int, [vp, vp, i64]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

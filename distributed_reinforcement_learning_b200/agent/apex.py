@@ -10,13 +10,14 @@ values -- so the learner branch of ``train_apex.py:82-155`` runs on it unchanged
   Agent.get_td_error          agent/apex.py:116-133
   Agent.distributed_train     agent/apex.py:135-154 -> (loss, td_error)
   Agent.train                 agent/apex.py:156-168
+  Agent.make_device_replay    (new) buffer_queue.Memory + the learner calls around it, kept on the GPU
 """
 import os
 import threading
 
 import numpy as np
 
-from ..apex_learner import MAIN, TARGET, NativeApexLearner
+from ..apex_learner import MAIN, TARGET, NativeApexLearner, NativeApexReplay
 from ..model import apex_value
 
 _AGENTS = {}
@@ -47,6 +48,7 @@ class Agent:
         self._engine = None
         self._slot = 0
         self._last = {}
+        self._replay = None
         self._lock = threading.RLock()   # actor threads sync from / act on this agent while the learner thread trains
         _AGENTS[model_name] = self
 
@@ -179,6 +181,9 @@ class Agent:
 
     def _train(self, state, next_state, previous_action, action, reward, done, is_weight):
         st = self._u8(np.stack(state))
+        if self._replay is not None and self._engine.B != st.shape[0]:
+            raise ValueError("a device replay of batch %d is attached: training on %d transitions would rebuild the "
+                             "learner under it" % (self._engine.B, st.shape[0]))
         if self._engine is not None and self._engine.B != st.shape[0]:
             self._pull_state()
             self._engine.close()
@@ -199,10 +204,68 @@ class Agent:
         """agent/apex.py:156-168 (unit importance weights; returns None like the reference)."""
         self._train(state, next_state, previous_action, action, reward, done, None)
 
+    def make_device_replay(self, capacity, batch_size, seed=0):
+        """(new) A prioritized replay of `capacity` transitions in this learner's GPU memory, trained on in minibatches
+        of `batch_size`.  Its ``add`` replaces get_td_error + the Memory.add loop, its ``train`` replaces Memory.sample +
+        distributed_train + the Memory.update loop (train_apex.py:106-155)."""
+        with self._lock:
+            if self._replay is not None:
+                raise RuntimeError("this agent already has a device replay; close it first")
+            if self._engine is not None and self._engine.B != int(batch_size):
+                self._pull_state()
+                self._engine.close()
+                self._engine = None
+            eng = self._get_engine(int(batch_size))
+            self._replay = DeviceReplay(self, NativeApexReplay(eng, capacity, seed))
+            return self._replay
+
     learning_rate = property(lambda self: self._last.get("learning_rate"))
     grad_norm = property(lambda self: self._last.get("grad_norm"))
     value_loss = property(lambda self: self._last.get("loss"))
     num_env_frames = property(lambda self: self._last.get("step", (self._opt or {}).get("step", 0)))
+
+
+class DeviceReplay:
+    """What Agent.make_device_replay returns: the learner loop of train_apex.py:106-155 over a replay in GPU memory.
+
+        replay.add(state, next_state, previous_action, action, reward, done)   # get_td_error + Memory.add, per record
+        loss, td_error = replay.train()     # Memory.sample -> distributed_train -> Memory.update
+    """
+
+    def __init__(self, agent, native):
+        self._agent, self.native = agent, native
+
+    def add(self, state, next_state, previous_action, action, reward, done):
+        with self._agent._lock:
+            self.native.add(self._agent._u8(np.stack(state)), self._agent._u8(np.stack(next_state)),
+                            np.asarray(previous_action), np.asarray(action), np.asarray(reward), np.asarray(done))
+
+    def train(self):
+        """-> (loss, td_error [batch]) of one step on a prioritized minibatch; the sampled priorities are updated."""
+        a = self._agent
+        with a._lock:
+            slot = a._slot
+            a._slot = (a._slot + 1) % self.native.learner.num_slots
+            out, td = self.native.step(slot)
+            a._last = out
+            return out["loss"], td
+
+    def __len__(self):
+        return len(self.native)
+
+    def total(self):
+        """SumTree.total (buffer_queue.py:348-349)."""
+        return self.native.info()["total"]
+
+    @property
+    def beta(self):
+        return self.native.info()["beta"]
+
+    def close(self):
+        with self._agent._lock:
+            self.native.close()
+            if self._agent._replay is self:
+                self._agent._replay = None
 
 
 def _locked(fn):

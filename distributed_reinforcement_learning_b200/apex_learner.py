@@ -80,3 +80,75 @@ class NativeApexLearner(dp.AdamLearner):
         N.check(N.lib.drl_apex_taps(self._h, *[N.ptr(a) for a in out]))
         return dict(main_q=out[0], next_main_q=out[1], target_q=out[2], target_value=out[3],
                     state_action_value=out[4])
+
+
+class NativeApexReplay:
+    """Prioritized replay of ``learner`` kept in its GPU memory (``drl_apex_replay_*``): ``buffer_queue.Memory`` and the
+    transitions it indexes.  ``add`` is ``Agent.get_td_error`` + ``Memory.add`` for any number of transitions;
+    ``step(slot)`` is ``Memory.sample`` -> ``distributed_train`` -> ``Memory.update`` as one enqueue on the learner's
+    stream, returning what ``learner.step`` returns.  The uniforms of the stratified draw come from a counter-based
+    generator seeded with ``seed`` (oracle/replay_np.py restates it).  Close the replay before its learner."""
+
+    def __init__(self, learner, capacity, seed=0):
+        self.learner = learner
+        self.B = learner.B
+        self.capacity = int(capacity)
+        self._r = C.c_void_p()
+        N.check(N.lib.drl_apex_replay_create(learner._h, self.capacity, C.c_uint64(int(seed)), C.byref(self._r)))
+
+    def close(self):
+        if getattr(self, "_r", None) is not None and self._r.value:
+            N.lib.drl_apex_replay_destroy(self._r)
+            self._r = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def add(self, state, next_state, previous_action, action, reward, done):
+        """n transitions, in chunks of the learner's batch (as Agent.get_td_error) -> their |td| are the priorities."""
+        n = int(np.asarray(state).shape[0])
+        for lo in range(0, n, self.B):
+            hi = min(lo + self.B, n)
+            arrs = self.learner._arrays(hi - lo, np.asarray(state)[lo:hi], np.asarray(next_state)[lo:hi],
+                                        np.asarray(previous_action)[lo:hi], np.asarray(action)[lo:hi],
+                                        np.asarray(reward)[lo:hi], np.asarray(done)[lo:hi])
+            N.check(N.lib.drl_apex_replay_add(self._r, hi - lo, *[N.ptr(a) for a in arrs]))
+
+    def step_async(self, slot=0):
+        N.check(N.lib.drl_apex_replay_step_async(self._r, int(slot)))
+
+    def step(self, slot=0):
+        """-> (scalars dict, td_error [B]) like NativeApexLearner.step."""
+        self.step_async(slot)
+        return self.learner.wait()
+
+    def last_sample(self):
+        ti, di = np.empty(self.B, np.int64), np.empty(self.B, np.int64)
+        pr, w = np.empty(self.B, np.float64), np.empty(self.B, np.float64)
+        N.check(N.lib.drl_apex_replay_last_sample(self._r, N.ptr(ti), N.ptr(di), N.ptr(pr), N.ptr(w)))
+        return dict(tree_index=ti, data_index=di, priority=pr, is_weight=w)
+
+    def last_update(self):
+        """-> (leaves, priorities) of the most recent add or post-step update, in call order."""
+        leaf, p = np.empty(self.B, np.int64), np.empty(self.B, np.float64)
+        cnt = C.c_int32()
+        N.check(N.lib.drl_apex_replay_last_update(self._r, N.ptr(leaf), N.ptr(p), self.B, C.byref(cnt)))
+        return leaf[:cnt.value].copy(), p[:cnt.value].copy()
+
+    def info(self):
+        n, w, dr = C.c_int64(), C.c_int64(), C.c_int64()
+        t, b = C.c_double(), C.c_double()
+        N.check(N.lib.drl_apex_replay_info(self._r, C.byref(n), C.byref(w), C.byref(t), C.byref(b), C.byref(dr)))
+        return dict(n_entries=int(n.value), write=int(w.value), total=float(t.value), beta=float(b.value),
+                    draws=int(dr.value))
+
+    def tree(self):
+        a = np.empty(2 * self.capacity - 1, np.float64)
+        N.check(N.lib.drl_apex_replay_read_tree(self._r, N.ptr(a), a.size))
+        return a
+
+    def __len__(self):
+        return self.info()["n_entries"]

@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(CSRC, "libdrl_b200.so")
 SOURCES = ["learner.cu", "layers.cu", "apex.cu", "r2d2.cu", "elementwise.cu", "vtrace.cu", "optimizer.cu", "ring.cu", "per.cu", "debug.cu",
-           "peer.cu"]
+           "peer.cu", "replay.cu"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 

@@ -1,8 +1,9 @@
 // adam_learner.cuh -- the host-side handle shell of the learners that train with TF1 Adam and keep a target network:
 // Ape-X and A3C (apex.cu) and R2D2 (r2d2.cu).  It owns the streams and events, the main / target parameters, the Adam
 // state, the gradient bucket, the mapped pinned result rows, the staging-slot handshake and the step lifecycle with its
-// CUDA graph cache.  A family handle derives from AdamLearner and adds its layout `pl`, its `cfg` (device, num_slots,
-// use_cuda_graph), its slot payloads and its forward + loss + backward enqueue (FwdBwd); the shell appends the update.
+// CUDA graph cache (run_step; run_filled_step for slots filled on the device).  A family handle derives from
+// AdamLearner and adds its layout `pl`, its `cfg` (device, num_slots, use_cuda_graph), its slot payloads and its
+// forward + loss + backward enqueue (FwdBwd); the shell appends the update.
 #pragma once
 #include <string>
 
@@ -367,6 +368,48 @@ int run_step(H* h, int slot, FwdBwd<H> fwd_bwd) {
   h->last_rows = h->B;
   h->last_slot = slot;
   DRL_CUDA_CHECK(cudaEventRecord(h->sync[slot].consumed, h->compute));
+  return record_step_end(h);
+}
+
+// run_step for a slot that device work fills instead of an H2D copy (the device replay, replay.cu): fill() runs on the
+// compute stream after any pending H2D into the slot, then the step, then after().  With use_cuda_graph all three are
+// captured into graphs[slot], a cache the caller owns.  The eager pass before capture is forward + loss + backward
+// only, so fill() and after() -- which advance the caller's state -- run exactly once per step, captured or not.  The
+// slot is left "not staged": a plain step on it needs a new stage first.
+template <class H, class Fill, class After>
+int run_filled_step(H* h, int slot, FwdBwd<H> fwd_bwd, std::vector<cudaGraphExec_t>& graphs, Fill&& fill,
+                    After&& after) {
+  DRL_TRY(check_slot(h, slot));
+  if ((int)graphs.size() < h->cfg.num_slots) graphs.resize(h->cfg.num_slots, nullptr);
+  SlotSync& s = h->sync[slot];
+  DRL_CUDA_CHECK(cudaStreamWaitEvent(h->compute, s.staged, 0));
+  pdl_break(h->compute);
+  if (h->cfg.use_cuda_graph) DRL_TRY(refresh_target_images(h));
+  DRL_CUDA_CHECK(cudaEventRecord(h->ev_start, h->compute));
+  h->main_images_stale = true;
+  int cnt = 0;
+  auto whole = [&]() -> int {
+    DRL_TRY(fill());
+    DRL_TRY(enqueue_step(h, slot, fwd_bwd, &cnt));
+    return after();
+  };
+  if (h->cfg.use_cuda_graph) {
+    if (!graphs[slot]) {
+      DRL_TRY(fwd_bwd(h, slot, nullptr));
+      h->main_images_stale = true;
+      DRL_TRY(capture_graph(h->compute, &graphs[slot], whole));
+      h->launches = cnt;
+    }
+    DRL_CUDA_CHECK(cudaGraphLaunch(graphs[slot], h->compute));
+  } else {
+    DRL_TRY(whole());
+    h->launches = cnt;
+  }
+  h->main_images_stale = true;
+  h->last_rows = h->B;
+  h->last_slot = slot;
+  DRL_CUDA_CHECK(cudaEventRecord(s.consumed, h->compute));
+  s.has_data = false;
   return record_step_end(h);
 }
 

@@ -8,6 +8,7 @@
 // through the same gather-GEMM kernels (layer_defs.cuh); the two streams of the dueling head share their input
 // concat = [a3 | emb(prev_a)] (K = 3392), so their first layers are one split-K GEMM with N = 2 x 256.
 #include "adam_learner.cuh"
+#include "replay.cuh"
 
 namespace drl {
 
@@ -448,6 +449,7 @@ struct drl_apex : AdamLearner {
   int a3c_clip = 0;
   float* adv = nullptr;        // [B] advantage tap
   std::vector<ApexSlot> slots; // payloads of AdamLearner::sync
+  int replays = 0;             // device replays attached to this handle (replay.cu)
 };
 
 namespace {
@@ -545,6 +547,65 @@ int stage_into(drl_apex* h, ApexSlot& s, cudaStream_t stream, int n, int row2, c
 
 }  // namespace
 
+// ---- the device replay's view of the handle (replay.cuh) -------------------------------------------------------
+namespace drl {
+
+int apex_replay_link(drl_apex* h, ApexReplayLink* out) {
+  out->mu = &h->mu;
+  out->device = h->cfg.device;
+  out->B = h->B;
+  out->algo = h->algo;
+  out->compute = h->compute;
+  out->td_dev = h->td_dev;
+  return DRL_OK;
+}
+
+void apex_replay_attach(drl_apex* h, int delta) {
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  h->replays += delta;
+}
+
+int apex_enqueue_td_error(drl_apex* h, int n, const uint8_t* state, const uint8_t* next_state,
+                          const int32_t* previous_action, const int32_t* action, const float* reward,
+                          const uint8_t* done, ApexRecordView* scratch) {
+  ApexSlot& s = h->slots[h->cfg.num_slots];      // scratch slot
+  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
+  // rows [0, n) = s, rows [n, 2n) = s' (packed, so that one main-network forward covers both)
+  DRL_TRY(stage_into(h, s, h->compute, n, n, state, next_state, previous_action, action, reward, done, nullptr));
+  pdl_break(h->compute);
+  const Streams st = streams_of(h);
+  DRL_TRY(apex_forward(st, h->pl, h->params, h->wi, s.frames, s.pa2, h->act, 2 * n, h->mode, h->main_images_stale,
+                       h->main_images_stale, false, nullptr));
+  h->main_images_stale = false;
+  DRL_TRY(apex_forward(st, h->pl, h->target, h->twi, s.frames + (size_t)n * Geo::FRAME, s.pa2 + n, h->tact, n, h->mode,
+                       h->target_images_stale, false, true, nullptr));
+  h->target_images_stale = false;
+  TdArgs a{};
+  a.vstream = h->act.vstream; a.mstream = h->act.mstream;
+  a.tvstream = h->tact.vstream; a.tmstream = h->tact.mstream;
+  a.action = s.pa2 + n; a.reward = s.reward; a.done = s.done; a.weight = nullptr;
+  a.discount = h->cfg.discount_factor; a.clip = (h->cfg.reward_clipping == DRL_REWARD_ABS_ONE) ? 1 : 0;
+  a.n = n; a.A = h->A;
+  a.main_q = h->main_q; a.next_main_q = h->next_main_q; a.target_q = h->target_q;
+  a.target_value = h->target_value; a.sav = h->sav; a.td_dev = h->td_dev; a.td_host = nullptr;
+  DRL_CUDA_CHECK((launch_k(apex_td_kernel, 1, 256, 0, h->compute, a)));
+  pdl_break(h->compute);
+  h->last_rows = n;
+  *scratch = ApexRecordView{s.frames, s.pa2, s.reward, s.done, s.weight, n};
+  return DRL_OK;
+}
+
+int apex_replay_step(drl_apex* h, int slot, std::vector<cudaGraphExec_t>& graphs, const ApexSlotWork& fill,
+                     const ApexSlotWork& after) {
+  DRL_TRY(check_slot(h, slot));
+  const ApexSlot& sl = h->slots[slot];
+  const ApexRecordView v{sl.frames, sl.pa2, sl.reward, sl.done, sl.weight, h->B};
+  return run_filled_step(h, slot, forward_backward, graphs, [&] { return fill(h->compute, v); },
+                         [&] { return after(h->compute, v); });
+}
+
+}  // namespace drl
+
 extern "C" {
 
 int drl_apex_create(const drl_apex_config* cfg, drl_apex** out) {
@@ -614,7 +675,13 @@ int drl_apex_create(const drl_apex_config* cfg, drl_apex** out) {
   return finish_create(h, rc, out);
 }
 
-int drl_apex_destroy(drl_apex* h) { return destroy_shell(h); }
+int drl_apex_destroy(drl_apex* h) {
+  if (h && h->replays > 0) {
+    set_error("destroy: %d device replay(s) still use this learner; destroy them first", h->replays);
+    return DRL_ERR_STATE;
+  }
+  return destroy_shell(h);
+}
 
 int drl_apex_param_count(const drl_apex* h, int64_t* n) {
   DRL_ENTER(h);
@@ -701,30 +768,10 @@ int drl_apex_td_error(drl_apex* h, int32_t n, const uint8_t* state, const uint8_
   DRL_ENTER(h);
   if (n < 1 || n > h->B) { set_error("td_error: n must be in [1, %d]", h->B); return DRL_ERR_INVALID; }
   if (!state || !next_state || !previous_action || !action || !reward || !done || !td_error) { set_error("td_error: null pointer"); return DRL_ERR_INVALID; }
-  ApexSlot& s = h->slots[h->cfg.num_slots];      // scratch slot
-  DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  // rows [0, n) = s, rows [n, 2n) = s' (packed, so that one main-network forward covers both)
-  DRL_TRY(stage_into(h, s, h->compute, n, n, state, next_state, previous_action, action, reward, done, nullptr));
-  pdl_break(h->compute);
-  const Streams st = streams_of(h);
-  DRL_TRY(apex_forward(st, h->pl, h->params, h->wi, s.frames, s.pa2, h->act, 2 * n, h->mode, h->main_images_stale,
-                       h->main_images_stale, false, nullptr));
-  h->main_images_stale = false;
-  DRL_TRY(apex_forward(st, h->pl, h->target, h->twi, s.frames + (size_t)n * Geo::FRAME, s.pa2 + n, h->tact, n, h->mode,
-                       h->target_images_stale, false, true, nullptr));
-  h->target_images_stale = false;
-  TdArgs a{};
-  a.vstream = h->act.vstream; a.mstream = h->act.mstream;
-  a.tvstream = h->tact.vstream; a.tmstream = h->tact.mstream;
-  a.action = s.pa2 + n; a.reward = s.reward; a.done = s.done; a.weight = nullptr;
-  a.discount = h->cfg.discount_factor; a.clip = (h->cfg.reward_clipping == DRL_REWARD_ABS_ONE) ? 1 : 0;
-  a.n = n; a.A = h->A;
-  a.main_q = h->main_q; a.next_main_q = h->next_main_q; a.target_q = h->target_q;
-  a.target_value = h->target_value; a.sav = h->sav; a.td_dev = h->td_dev; a.td_host = nullptr;
-  DRL_CUDA_CHECK((launch_k(apex_td_kernel, 1, 256, 0, h->compute, a)));
+  ApexRecordView scratch{};
+  DRL_TRY(apex_enqueue_td_error(h, n, state, next_state, previous_action, action, reward, done, &scratch));
   DRL_CUDA_CHECK(cudaMemcpyAsync(td_error, h->td_dev, (size_t)n * 4, cudaMemcpyDeviceToHost, h->compute));
   DRL_CUDA_CHECK(cudaStreamSynchronize(h->compute));
-  h->last_rows = n;
   return DRL_OK;
 }
 

@@ -1,7 +1,8 @@
 // per.cu -- prioritized replay index behind drl_per_* (include/drl_b200.h): the host-side sum tree of
-// buffer_queue.SumTree / Memory (distributed_queue/buffer_queue.py:326-416).  Host code only (the transitions stay
-// with the caller; what the learner needs from here per step are B tree walks and B leaf updates, microseconds of
-// pointer chasing that belong next to the Python loop, not on the GPU).  The tree is float64 and every update adds
+// buffer_queue.SumTree / Memory (distributed_queue/buffer_queue.py:326-416).  Host code only: the transitions stay
+// with the caller, as in the reference's loop, which this path serves unchanged (B tree walks and B leaf updates per
+// step next to the Python loop).  A learner that keeps the transitions on the GPU uses the device replay instead
+// (replay.cu, drl_apex_replay_*), whose tree kernels follow the same arithmetic.  The tree is float64 and every update adds
 // the same `change` to the same ancestors in the same order as the reference's recursion, so totals, sampled
 // indices and priorities are bit-identical to the NumPy implementation for the same uniform draws.
 #include <math.h>

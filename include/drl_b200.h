@@ -387,6 +387,48 @@ int drl_per_size(const drl_per* p, int64_t* n_entries);  /* SumTree.n_entries */
 int drl_per_beta(const drl_per* p, double* beta);
 
 /* ------------------------------------------------------------------------------------------
+ * (new) Device-resident prioritized replay of an Ape-X learner: buffer_queue.Memory / SumTree together with the
+ * transitions themselves (distributed_queue/buffer_queue.py:326-416), kept in the learner's GPU memory.  Storage is
+ * field-major (state / next_state [cap, H*W*C] u8, previous_action / action [cap] i32, reward [cap] f32, done [cap]
+ * u8); the sum tree is 2*cap - 1 float64 nodes with the leaves last, updated with the reference's arithmetic order
+ * (totals bit-identical to drl_per_* for the same leaf values).  Sampling draws its uniforms on the device: Philox4x32-10
+ * with key (seed lo, seed hi) and counter (stratum, draw call lo, draw call hi, 0), u = ((x0 << 32 | x1) >> 11) * 2^-53;
+ * the draw call counter advances by one per sample.  Priorities are (|td| + 0.001)^0.6 with CUDA's double pow (within
+ * a few ulp of glibc's).  The replay runs on the learner's streams and takes its lock; drl_apex_destroy refuses
+ * (DRL_ERR_STATE) while a replay of the learner is alive.  The host drl_per_* path is unchanged.
+ * ------------------------------------------------------------------------------------------ */
+typedef struct drl_apex_replay drl_apex_replay;
+/* Memory.__init__ (buffer_queue.py:378-381) on the learner's device, zero-initialised, beta 0.4.  capacity >= 2;
+ * DRL_ERR_INVALID for an A3C handle; DRL_ERR_CUDA (with the byte count) when the storage does not fit. */
+int drl_apex_replay_create(drl_apex* h, int64_t capacity, uint64_t seed, drl_apex_replay** out);
+int drl_apex_replay_destroy(drl_apex_replay* r);
+/* learner.get_td_error + Memory.add for n <= batch transitions (train_apex.py:106-122, buffer_queue.py:386-388): the
+ * same forward and |td| as drl_apex_td_error, then the rows are copied at the write cursor (wrapping) and their leaves
+ * set in call order.  Synchronous: the host buffers are free on return.  Shapes as drl_apex_stage. */
+int drl_apex_replay_add(drl_apex_replay* r, int32_t n, const uint8_t* state, const uint8_t* next_state,
+                        const int32_t* previous_action, const int32_t* action, const float* reward,
+                        const uint8_t* done);
+/* Memory.sample -> distributed_train -> Memory.update (train_apex.py:129-155) as ONE enqueue on the learner's compute
+ * stream: sample batch strata, gather them into training slot `slot` (float32 importance weights included), the
+ * learner step, then the new priorities of the sampled leaves from the step's |td|.  Collect with drl_apex_wait.  The
+ * slot is left unstaged (a plain drl_apex_step on it needs a new drl_apex_stage).  DRL_ERR_STATE on an empty replay. */
+int drl_apex_replay_step_async(drl_apex_replay* r, int32_t slot);
+int drl_apex_replay_step(drl_apex_replay* r, int32_t slot, drl_apex_out* out, float* td_error);
+/* Inspection: the most recent sample's [batch] tree indices, data indices, priorities and float64 weights
+ * (Memory.sample's idxs / is_weight); any pointer may be NULL. */
+int drl_apex_replay_last_sample(drl_apex_replay* r, int64_t* tree_index, int64_t* data_index, double* priority,
+                                double* is_weight);
+/* Inspection: the (leaf, priority) list of the most recent add or post-step update, in call order (*count entries,
+ * at most max_count copied). */
+int drl_apex_replay_last_update(drl_apex_replay* r, int64_t* leaf, double* priority, int32_t max_count,
+                                int32_t* count);
+/* Inspection: SumTree.n_entries / write, SumTree.total (:348-349), Memory.beta and the draw calls so far. */
+int drl_apex_replay_info(drl_apex_replay* r, int64_t* n_entries, int64_t* write, double* total, double* beta,
+                         int64_t* draws);
+/* Inspection: all 2*capacity - 1 tree nodes (count must equal that). */
+int drl_apex_replay_read_tree(drl_apex_replay* r, double* host_nodes, int64_t count);
+
+/* ------------------------------------------------------------------------------------------
  * R2D2 learner (SURVEY.md section 8(f) row 3, BASELINE.json config 5): replaces r2d2.Agent's learner graph
  * (agent/r2d2.py:13-95) over model/r2d2_lstm.py:28-116 (conv stack + action embedding + ONE LSTMCell, unrolled seq_len
  * steps per scope from a stored (h, c) with the carried state multiplied by (1 - done) after every step; dense 128;
